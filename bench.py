@@ -46,6 +46,8 @@ DPX_LANES_PER_CLK_PER_SM = 64       # measured: tools/microbench/pipe_rates.cu -
 DPX_INSTR_PER_CELL = 6              # 32-bit word: 2 (five-way max + floor for H) + 4 (E1, E2, F1, F2 updates)
 DPX_INSTR_PER_CELL_PAIR = 7         # u16x2 words (two cells per instruction): 3 for H (no .RELU on unsigned halves) + 4
 HEADLINE = "config 2: HTT CAG/CCG amplicon, 5k ONT reads, two BED rows, rounds 1-3"
+DUMP_MAX_BYTES = 64_000_000         # --dump-outputs in all, headers included; above it a seeded sample of reads is written
+NPY_HEADER_BYTES = 128              # header of a 1-D .npy file (format 1.0)
 
 
 def load_peaks():
@@ -288,6 +290,25 @@ class Workload:
         return checked
 
 
+def dump_outputs(out_dir, arrays):
+    """arrays: name -> one value per read, all of the same length -> out_dir/<name>.npy as float64, and the reads'
+    positions in read_index.npy.  Above DUMP_MAX_BYTES in all, every file holds the same seeded sample of the reads."""
+    os.makedirs(out_dir, exist_ok=True)
+    n = len(next(iter(arrays.values())))
+    n_files = len(arrays) + 1
+    keep = (DUMP_MAX_BYTES - NPY_HEADER_BYTES * n_files) // (8 * n_files)
+    idx = np.arange(n) if n <= keep else np.sort(np.random.default_rng(0).choice(n, keep, replace=False))
+    np.save(os.path.join(out_dir, "read_index.npy"), idx.astype(np.float64))
+    for name, a in arrays.items():
+        a = np.asarray(a, dtype=np.float64)
+        assert len(a) == n, (name, len(a), n)
+        np.save(os.path.join(out_dir, name + ".npy"), a[idx])
+
+
+def sizes_or_nan(rrs, attr):
+    return [np.nan if v is None else float(v) for rr in rrs for v in (getattr(rd, attr) for rd in rr.read_dict.values())]
+
+
 def kernel_table(linfo, kern_ms, launches, peak16, peak32):
     """Per-kernel rooflines from nr_batch_launch_info: executed cells per launch / mean CUDA-event time per launch."""
     names = [("pair_round2_kernel (round 2, u16x2 pairs + 32-bit entries beside them)", 0, "paired"),
@@ -375,6 +396,7 @@ def time_e2e(wl, torch, passes_total):
                 continue     # buffers that an earlier, differently interleaved pass never asked for (a one-off 100 ms)
             total += dt
             wl.e2e_pass_ms.append(round(dt * 1e3, 3))
+            wl.last_rrs = rrs
     finally:
         gc.unfreeze()
     return total
@@ -546,7 +568,9 @@ def measure_phasing(torch, engine, n_loci=2000, reads_per_locus=30, n_cpu=6):
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=20)
+    ap.add_argument("--steps", type=int, default=20,
+                    help="timed steps of `value` (each --passes passes over the batch); the end-to-end and C-ABI legs time "
+                         "as many passes, the per-kernel event leg a quarter as many steps (at least one)")
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="b200", choices=["b200", "reference"])
     ap.add_argument("--reads", type=int, default=5000, help="reads in the headline batch (config 2: 5000)")
@@ -556,6 +580,9 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-configs", action="store_true", help="skip the other four configs and the strong-scaling leg")
     ap.add_argument("--no-flush", action="store_true", help="no L2 flush between steps (for ncu traffic captures)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the headline batch's results of the last timed step (and of the last e2e pass) as "
+                         "DIR/<name>.npy, one float64 value per read, so that two builds can be compared (rank 0)")
     args = ap.parse_args()
 
     rank = int(os.environ.get("RANK", "0"))
@@ -563,6 +590,8 @@ def main():
     world = int(os.environ.get("WORLD_SIZE", "1"))
 
     if args.impl == "reference":
+        if args.dump_outputs:
+            ap.error("--dump-outputs writes the GPU arm's results; --impl reference has none")
         run_reference_arm(args, rank)
         return
 
@@ -603,16 +632,19 @@ def main():
     dev_ms = time_resident_async(wl, torch, stream, flush, K, P)                 # the number `value` is made of
     barrier()
     wall = time.perf_counter() - wall0
-    ev_ms, kern_ms = time_resident(wl, torch, stream, flush, max(2, K // 4), P, engine)      # per-kernel event times
+    if args.dump_outputs:
+        r2_score, r2_tend, r2_starts = wl.b2.fetch_round2()
+        r3_sum_k, r3_n_k, r3_top = wl.b3.fetch_round3()
+    ev_ms, kern_ms = time_resident(wl, torch, stream, flush, max(1, K // 4), P, engine)      # per-kernel event times
     linfo = [wl.b2.launch_info(), wl.b3.launch_info()]
-    n_ev = max(2, K // 4) * P
+    n_ev = max(1, K // 4) * P
     # the 100 ms clock poll covers the device-timed region above and stops here: every NVML query stalls the CUDA calls
     # of this process for a while, which a host-timed 6 ms pass feels (measured: +0.8 ms per pass under the poll); the e2e
     # passes get one clock reading before and one after instead
     clocks = sampler.stop()
     clocks["e2e_before"] = clock_snapshot(local_rank)
     # e2e through the operator API
-    e2e_passes = max(K, 10)
+    e2e_passes = K
     for _ in range(2):
         wl.e2e_pass(wl.fresh())
     barrier()
@@ -621,6 +653,11 @@ def main():
     barrier()
     clocks["e2e_after"] = clock_snapshot(local_rank)
     total_ms = float(sum(dev_ms))
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, {
+            "round2_score": r2_score, "round2_tend": r2_tend, "round2_starts_by_left": r2_starts,
+            "round3_sum_k": r3_sum_k, "round3_n_k": r3_n_k, "round3_top_score": r3_top,
+            **{f"e2e_{a}": sizes_or_nan(wl.last_rrs, a) for a in ("round1_repeat_size", "round2_repeat_size", "round3_repeat_size")}})
 
     # resumed round 3 (from round 2's kept state) == a fresh round-3 batch (full forward sweeps): checked on every run
     s3 = wl.b3.fetch_round3()

@@ -12,42 +12,60 @@ import numpy as np
 import pytest
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-REF_SRC = "/root/reference/src"
+# the original NanoRepeat's src/ directory; it is not part of this repository: given, the boundary shape stored under
+# tests/golden is re-checked against it and the shim runs under the reference's own round functions
+REF_SRC = os.environ.get("NANOREPEAT_REFERENCE_SRC", "")
+NO_REF = "needs the original NanoRepeat sources: set NANOREPEAT_REFERENCE_SRC to its src/ directory"
 
 
 def _import_reference_module():
-    """NanoRepeat.nanoRepeat_bam from /root/reference with its absent third-party imports stubbed (build container only)."""
+    """NanoRepeat.nanoRepeat_bam from REF_SRC with its absent third-party imports stubbed."""
+    sys.path.insert(0, REF_SRC)
     sys.path.insert(0, os.path.join(ROOT, "tests", "golden"))
     import make_golden
     return make_golden.import_reference()
 
 
-@pytest.mark.skipif(not os.path.isdir(REF_SRC), reason="the reference tree exists in the build container only")
 def test_install_matches_the_reference_module_shape():
     """install() patches exactly the names quantify1repeat_from_bam calls, with the reference's parameter lists; the
-    reference's own Read / RepeatRegion carry every attribute the operators read or write."""
+    package's Read / RepeatRegion carry every attribute the operators read or write, with the reference's defaults
+    (tests/golden/boundary_shape.json).  With the reference sources given, the stored shape is re-derived from them and
+    install() is run on the reference's own module as well."""
+    import types
     import nanorepeat_b200 as nrb
-    ref_bam, ref_rr = _import_reference_module()
-    own = {n: getattr(ref_bam, n) for n in ("round1_and_round2_estimation", "round3_estimation")}
-    try:
-        nrb.install(ref_bam)
-        for name, fn in own.items():
-            assert getattr(ref_bam, name) is getattr(nrb, name)
-            assert list(inspect.signature(fn).parameters) == list(inspect.signature(getattr(nrb, name)).parameters), name
-        src = inspect.getsource(ref_bam.quantify1repeat_from_bam)
-        assert "round1_and_round2_estimation(" in src and "round3_estimation(" in src      # looked up in module globals
-    finally:
-        for name, fn in own.items():
-            setattr(ref_bam, name, fn)
-    rd, rr = ref_rr.Read(), ref_rr.RepeatRegion()
-    for attr in ("dist_between_anchors", "round1_repeat_size", "round2_repeat_size", "round3_repeat_size"):
-        assert hasattr(rd, attr) and getattr(rd, attr) is None
-    for attr in ("left_anchor_seq", "right_anchor_seq", "repeat_unit_seq", "read_dict", "read_core_seq_dict"):
-        assert hasattr(rr, attr)
+    from conftest import load_golden
+    want = load_golden("boundary_shape")
+    del want["source"]
+    assert set(want["quantify1repeat_from_bam_calls"]) == set(want["signatures"])       # looked up in module globals
+    modules = [types.ModuleType("nanoRepeat_bam")]
+    if os.path.isdir(REF_SRC):
+        ref_bam, ref_rr = _import_reference_module()
+        import make_golden_boundary
+        assert make_golden_boundary.shape(ref_bam, ref_rr) == want
+        pickle.dumps(ref_rr.RepeatRegion())
+        modules.append(ref_bam)
+    for mod in modules:
+        before = dict(vars(mod))
+        try:
+            nrb.install(mod)
+            changed = {n for n, v in vars(mod).items() if before.get(n, None) is not v}
+            assert changed == set(want["signatures"]), changed
+            for name, params in want["signatures"].items():
+                assert getattr(mod, name) is getattr(nrb, name)
+                assert list(inspect.signature(getattr(nrb, name)).parameters) == params, name
+        finally:
+            for name in want["signatures"]:
+                if name in before:
+                    setattr(mod, name, before[name])
+    rd, rr = nrb.Read(), nrb.RepeatRegion()
+    for attr in want["read_defaults_none"]:
+        assert hasattr(rd, attr) and getattr(rd, attr) is None, attr
+    for attr in want["repeat_region_attributes"]:
+        assert hasattr(rr, attr), attr
     pickle.dumps(rr)
 
 
-@pytest.mark.skipif(not os.path.isdir(REF_SRC), reason="the reference tree exists in the build container only")
+@pytest.mark.skipif(not os.path.isdir(REF_SRC), reason=NO_REF)
 def test_shim_feeds_the_unmodified_reference_functions(monkeypatch, tmp_path):
     """The reference's UNMODIFIED round1_and_round2_estimation / round3_estimation on top of pymm2_shim.main, with the
     engine call inside the shim answered by the oracle (no GPU here): the shim's file handling, command recognition and
@@ -79,6 +97,49 @@ def test_shim_feeds_the_unmodified_reference_functions(monkeypatch, tmp_path):
         rd = R.read_dict[name]
         assert (rd.round1_repeat_size, rd.round2_repeat_size) == (exp["r1"], exp["r2"])
         assert (None if rd.round3_repeat_size is None else float(rd.round3_repeat_size)) == exp["r3"]
+
+
+def test_shim_prints_the_paf_the_golden_fixtures_were_made_from(monkeypatch, tmp_path):
+    """The part of the test above that needs no reference sources: on the reference's round-2 command and, for every
+    read round 2 placed, its round-3 command over the ladder the reference builds (oracle/selection.ladder_bounds,
+    nanoRepeat_bam.py:463-472), pymm2_shim.main (engine call answered by the oracle) prints, line for line, the columns
+    the reference reads (query, target, target length, target start / end, AS) as the stand-in aligner whose PAF the
+    reference's functions turned into tests/golden/cfg1_small.json (tests/golden/make_golden.py).  Any other command
+    (Step 1's anchor search) is refused."""
+    from conftest import load_golden
+    from nanorepeat_b200 import pymm2_shim, engine
+    from oracle import nr_oracle, selection
+    sys.path.insert(0, os.path.join(ROOT, "tests", "golden"))
+    import make_golden
+    monkeypatch.setattr(engine, "get_preset", lambda dt: nr_oracle.scoring())
+    monkeypatch.setattr(engine, "score_tasks", lambda q, t, sc: nr_oracle.align_batch(q, t, sc, n_threads=nr_oracle.max_threads()))
+    doc = load_golden("cfg1_small")
+    reg = doc["regions"][0]
+    left, right, motif = reg["left"], reg["right"], reg["motif"]
+    r1_max = max(reg["dists"]) / len(motif)                                   # round-2 template, :339-355
+    T = int(r1_max * 1.5) + 1
+    if T < r1_max + 10:
+        T = int(r1_max + 10)
+    (tmp_path / "round1_ref.fasta").write_text(f">{T}\n{left}{motif * T}\n")
+    with open(tmp_path / "core_sequences.fastq", "w") as f:
+        for name, core in zip(reg["read_names"], reg["cores"]):
+            f.write(f"@{name}\n{core}\n+\n{'0' * len(core)}\n")
+    cmds = [f"-c -t 1 -x map-ont -f 0.0 {tmp_path}/round1_ref.fasta {tmp_path}/core_sequences.fastq"]
+    for i, (name, core, exp) in enumerate(zip(reg["read_names"], reg["cores"], reg["expected"])):
+        if exp["r2"] is None:
+            continue
+        kmin, kmax = selection.ladder_bounds(exp["r2"], doc["fast_mode"])
+        ladder = tmp_path / f"round3_reference.{kmin}-{kmax}.fasta"
+        ladder.write_text("".join(f">{k}\n{left}{motif * k}{right}\n" for k in range(kmin, kmax + 1)))
+        (tmp_path / f"round3_input.read{i}.fasta").write_text(f">{name}\n{core}\n")
+        cmds.append(f"-x map-ont -f 0.0 -N 100 -c --eqx -t 1 {ladder} {tmp_path}/round3_input.read{i}.fasta")
+    assert len(cmds) >= 4
+
+    def columns(paf):
+        return [[r[i] for i in (0, 5, 6, 7, 8, 12)] for r in (ln.split("\t") for ln in paf.splitlines())]
+    for cmd in cmds:
+        got, want = pymm2_shim.main(cmd)[0], make_golden.fake_pymm2_main(cmd)[0]
+        assert len(columns(got)) >= 2 and columns(got) == columns(want), cmd
     with pytest.raises(NotImplementedError):
         pymm2_shim.main("-c -t 4 -x map-ont anchors.fasta region.fastq")       # Step 1's command is not this library's
 
