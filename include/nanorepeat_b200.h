@@ -85,7 +85,8 @@ typedef struct nr_stats_t {
 
 /* How the last nr_batch_run split its work (bench.py: one roofline per kernel). */
 typedef struct nr_launch_info_t {
-    int64_t paired_cells;   /* DP cells the paired u16x2 launch updates (both halves of every word, padding included) */
+    int64_t paired_cells;   /* DP cells the paired u16x2 launch updates (both halves of every word, padding included);
+                               after a run of a round-2 batch: the cells it executed (the dominance exit skips some) */
     int64_t rest_cells;     /* DP cells of the 32-bit launch beside it (long reads, other scorings, ...) */
     int32_t n_pairs;        /* warps' worth of paired tasks */
     int32_t n_rest;         /* tasks of the 32-bit launch */
@@ -95,6 +96,8 @@ typedef struct nr_launch_info_t {
     float reserved2;
     int64_t paired_useful_cells;   /* the same counts without padding: only rows that belong to a read (a warp sweeps */
     int64_t rest_useful_cells;     /* 32 * R rows per pair / stripe whatever the reads' lengths) */
+    int64_t planned_paired_cells;          /* paired_cells and paired_useful_cells as planned: every pair sweeps its */
+    int64_t planned_paired_useful_cells;   /* whole template */
 } nr_launch_info_t;
 
 /* Data-type preset table (reference tk.py:502-517: ont, ont_sup, ont_q20, clr, hifi -- all map-ont). */

@@ -10,6 +10,7 @@
 #include "nr_launch.h"
 
 #include <algorithm>
+#include <numeric>
 #if defined(__x86_64__)
 #include <tmmintrin.h>
 #endif
@@ -325,6 +326,7 @@ struct nr_batch {
     int* h_spin = nullptr;                    // pinned: the kernels' give-up flag after the run (long reads only)
     long long paired_cells = 0, rest_cells = 0;
     long long paired_useful = 0, rest_useful = 0;   // the same without padding: rows of real reads only
+    bool round2_exit = false;                 // the single-stripe round-2 pairs may end their sweeps early (Pair2::check_col)
     size_t n_out = 0;                         // records in d_out / h_out
     std::vector<int32_t> order;               // entries of the 32-bit launch: (task << 7) | code (nr_kernels.cuh)
     std::vector<nr::CoopInfo> coop;           // scratch of the multi-stripe tasks
@@ -333,6 +335,7 @@ struct nr_batch {
     int32_t* d_coop_idx = nullptr;
     std::vector<int32_t> lt_src;              // round 3 over a round-2 batch's reads: that batch's task of every ladder task
     uint32_t* d_state = nullptr;              // round 2 pairs: DP state after column |left| - 2, kept for round 3
+    uint32_t* d_kept = nullptr;               // round 2 dominance exit: 128 words per warp of the launch
     size_t state_bytes = 0;
     int* d_flags = nullptr;                   // progress flags of the multi-stripe tasks, zeroed before every run
     size_t flags_bytes = 0;
@@ -437,6 +440,19 @@ bool is_map_ont(const nr_scoring_t& c) {
            c.ambiguous == 1;
 }
 
+// Round 2's dominance exit (nr_pair_kernels.cuh, Sweep::run; DESIGN.md section 4.9).  NR_ROUND2_EXIT=0 turns it off
+// for the batches committed while it is set (A/B measurements); it changes no result either way.
+bool round2_exit_enabled() {
+    const char* e = getenv("NR_ROUND2_EXIT");
+    return !(e && atoi(e) == 0);
+}
+// A core is 100 read bases of left flank + repeat + 100 of right flank (nanoRepeat_bam.py:308-316), so its repeat
+// ends near column |left| + q - 100 of the template and the DP past it turns periodic within a few motif copies.  On
+// config 2 (tools/round2_exit_census.py) the sweep ends at |left| + q - 83 on average; checks from |left| + q - 192 find
+// the same exits as checks from |left| on (18.1 % of the region's cells), from |left| + q - 100 they find 16.5 %.
+int round2_check_col(int n_left, int q_len) { return std::max(n_left + 1, n_left + q_len - 192); }
+int round2_predicted_exit(int n_left, int q_len) { return n_left + std::max(q_len - 64, 32); }
+
 // Pair up the eligible tasks of one region (ids[]: task indices, all of the same template): neighbours in read length
 // share a warp, one per 16-bit half of the DP words (nr_pair_kernels.cuh).  key(i) orders the tasks.
 template <class Key, class Emit>
@@ -503,11 +519,13 @@ int plan_batch(nr_batch* b) {
     trace.mark("task shapes");
     // ---- paired launch: two reads of one region per warp ----
     std::vector<long long> pair_cost;
+    std::vector<long long> deal_cost;     // round 2: the cost the pairs are dealt by, the sweep up to the predicted exit
     Launch& L = b->launch;
     L = {};
     long long state_off = 0;
     long long rung_off = 0;           // (P, J) token pairs of the paired ladders, single-stripe pairs first
     if (b->pair && fixed && !ladder && b->kind == KIND_ROUND2) {
+        const bool exits = round2_exit_enabled();
         for (const RegionInfo& g : b->regions) {
             std::vector<int> ids;
             for (int r = g.first_read; r < g.first_read + g.n_reads; ++r) {
@@ -516,7 +534,15 @@ int plan_batch(nr_batch* b) {
             }
             make_pairs(ids, [&](int i) { return b->tasks[i].q_len; }, [&](int x, int y) {
                 const int R = nr::pr::pair_rows(b->tasks[x].q_len);      // x is the longer read
-                nr::pr::Pair2 p = {x, y, g.n_left, -1};
+                nr::pr::Pair2 p = {x, y, g.n_left, -1, -1, 0, {0, 0}};
+                const int t_len = b->tasks[x].t_len;
+                int cols = t_len;
+                if (exits) {
+                    p.check_col = round2_check_col(g.n_left, b->tasks[x].q_len);
+                    p.period = 16 / std::gcd(16, g.motif_len) * g.motif_len;
+                    cols = std::min(t_len, round2_predicted_exit(g.n_left, b->tasks[x].q_len));
+                    b->round2_exit = true;
+                }
                 if (g.n_left >= 2 && state_off + nr::pr::state_words(R) < 0x7fffffffLL) {
                     p.state_off = (int32_t)state_off;                    // round 3 resumes from here (nr_batch_begin_round3_from)
                     state_off += nr::pr::state_words(R);
@@ -525,8 +551,9 @@ int plan_batch(nr_batch* b) {
                 paired[x] = 1;
                 if (y >= 0) paired[y] = 1;
                 L.pair_R = std::max(L.pair_R, R);
-                pair_cost.push_back((long long)32 * R * b->tasks[x].t_len);
-                b->paired_useful += (long long)(b->tasks[x].q_len + (y >= 0 ? b->tasks[y].q_len : 0)) * b->tasks[x].t_len;
+                pair_cost.push_back((long long)32 * R * t_len);
+                deal_cost.push_back((long long)32 * R * cols);
+                b->paired_useful += (long long)(b->tasks[x].q_len + (y >= 0 ? b->tasks[y].q_len : 0)) * t_len;
             });
         }
     } else if (b->pair && fixed && ladder && b->flag) {
@@ -596,7 +623,8 @@ int plan_batch(nr_batch* b) {
         std::vector<int> po(L.n_pairs);
         {
             std::vector<uint64_t> w(L.n_pairs);      // (cost << 24) | ~index: pair costs stay below 2^40, pairs below 2^24
-            for (int i = 0; i < L.n_pairs; ++i) w[i] = ((uint64_t)pair_cost[i] << 24) | (uint32_t)(0xffffff - i);
+            const std::vector<long long>& dc = deal_cost.empty() ? pair_cost : deal_cost;
+            for (int i = 0; i < L.n_pairs; ++i) w[i] = ((uint64_t)dc[i] << 24) | (uint32_t)(0xffffff - i);
             std::sort(w.begin(), w.end(), std::greater<uint64_t>());
             for (int i = 0; i < L.n_pairs; ++i) po[i] = 0xffffff - (int)(w[i] & 0xffffff);
         }
@@ -881,6 +909,8 @@ int plan_batch(nr_batch* b) {
     if (scratch_total && (rc = cached_alloc((void**)&b->d_scratch, b->scratch_bytes, BUF_SCRATCH))) return rc;
     if (b->flags_bytes && (rc = cached_alloc((void**)&b->d_flags, b->flags_bytes, BUF_DEV))) return rc;
     if (b->state_bytes && (rc = cached_alloc((void**)&b->d_state, b->state_bytes, BUF_DEV))) return rc;
+    if (b->round2_exit &&
+        (rc = cached_alloc((void**)&b->d_kept, sizeof(uint32_t) * 128 * kWarpsPerBlock * (size_t)g_ctx.sm_count, BUF_DEV))) return rc;
     if (b->flag) {
         b->sel_bytes = sizeof(int4) * std::max<size_t>((size_t)b->n_reads, 1);
         if ((rc = cached_alloc((void**)&b->d_sel, b->sel_bytes, BUF_DEV))) return rc;
@@ -1036,11 +1066,13 @@ int run_batch(nr_batch* b, cudaStream_t st) {
         if (getenv("NR_PLAIN_DEAL")) deal.nb_long = -1;      // tuning / debugging
         CUDA_TRY(mark(2, st));
         if (!ladder_batch) {
-            const int stride = exact_smem_int4(std::max(L.pair_R, L.R));
+            // the dominance exit keeps a cut (H, E1, E2 of every row) beside each pair's profile
+            const int stride = std::max(exact_smem_int4(std::max(L.pair_R, L.R)),
+                                        b->round2_exit ? exact_smem_int4(L.pair_R) + 3 * L.pair_R * 8 : 0);
             const size_t smem = (size_t)wpb * stride * sizeof(int4);
             if (smem > nrl::kMaxDynShared) return fail(NR_ERR_ARG, "launch needs %zu bytes of shared memory", smem);
             CUDA_TRY(nrl::launch_pair_round2(blocks, wpb * 32, smem, st, static_cast<const nr::pr::Pair2*>(b->d_pairs), deal, b->d_tasks,
-                                             ra, b->d_pool, k, b->d_counters, stride, b->d_out, b->d_state));
+                                             ra, b->d_pool, k, b->d_counters, stride, b->d_out, b->d_state, b->d_kept));
         } else {
             const int stride = pair_ladder_smem_int4(L.pair_R, L.R);
             const size_t smem = (size_t)wpb * stride * sizeof(int4);
@@ -1476,6 +1508,7 @@ void nr_batch_destroy(nr_batch_t* b) {
     cached_free(b->d_scratch, b->scratch_bytes, BUF_SCRATCH);
     cached_free(b->d_flags, b->flags_bytes, BUF_DEV);
     cached_free(b->d_state, b->state_bytes, BUF_DEV);
+    if (b->d_kept) cached_free(b->d_kept, sizeof(uint32_t) * 128 * kWarpsPerBlock * (size_t)g_ctx.sm_count, BUF_DEV);
     cached_free(b->d_sel, b->sel_bytes, BUF_DEV);
     cached_free(b->h_sel, b->sel_bytes, BUF_PIN);
     cached_free(b->d_prung, b->prung_bytes, BUF_DEV);
@@ -1748,14 +1781,20 @@ int nr_batch_launch_info(nr_batch_t* b, nr_launch_info_t* out) {
     if (!b || !out) return fail(NR_ERR_ARG, "nr_batch_launch_info: NULL argument");
     if (!b->committed) return fail(NR_ERR_ARG, "nr_batch_launch_info: batch was not committed");
     *out = {};
-    out->paired_cells = b->paired_cells;
+    out->paired_cells = out->planned_paired_cells = b->paired_cells;
     out->rest_cells = b->rest_cells;
-    out->paired_useful_cells = b->paired_useful;
+    out->paired_useful_cells = out->planned_paired_useful_cells = b->paired_useful;
     out->rest_useful_cells = b->rest_useful;
     out->n_pairs = b->launch.n_pairs;
     out->n_rest = b->launch.count;
     if (b->ran) {
         CUDA_TRY(cudaEventSynchronize(b->ev_done));
+        if (b->round2_exit) {       // what the dominance exit skipped in the last run (the counters stay until the next)
+            unsigned long long skipped[2];
+            CUDA_TRY(cudaMemcpy(skipped, b->d_counters + nr::pr::kExitSlot, sizeof(skipped), cudaMemcpyDeviceToHost));
+            out->paired_cells -= 2 * (int64_t)skipped[0];
+            out->paired_useful_cells -= (int64_t)(skipped[1] / 32);
+        }
         if (b->h_redo_count) out->n_redo = *b->h_redo_count;
         if (b->timed[0]) CUDA_TRY(cudaEventElapsedTime(&out->rest_ms, b->ev_t[0], b->ev_t[1]));
         if (b->timed[1]) CUDA_TRY(cudaEventElapsedTime(&out->paired_ms, b->ev_t[2], b->ev_t[3]));

@@ -18,7 +18,8 @@ cudaError_t launch_ladder(bool flag, int blocks, int threads, size_t smem, cudaS
                           const nr::LadderRegion* regs, const nr::ScoreW& k, int* counter, int stride, int4* out, int4* sel);
 cudaError_t launch_pair_round2(int blocks, int threads, size_t smem, cudaStream_t st, const nr::pr::Pair2* pairs,
                                const nr::pr::Deal& deal, const nr::Task* tasks, const nr::RestArgs& ra, const uint32_t* pool,
-                               const nr::ScoreW& k, int* counter, int stride, int4* out, uint32_t* state);
+                               const nr::ScoreW& k, int* counter, int stride, int4* out, uint32_t* state,
+                               uint32_t* kept);
 cudaError_t launch_pair_ladder(int blocks, int threads, size_t smem, cudaStream_t st, const nr::pr::Pair3* pairs,
                                const nr::pr::Deal& deal, const nr::LadderTask* tasks, const nr::RestArgs& ra,
                                const uint32_t* qpool, const uint32_t* pool, const nr::LadderRegion* regs, const nr::ScoreW& k,

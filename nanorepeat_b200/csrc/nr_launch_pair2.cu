@@ -5,7 +5,8 @@
 namespace nrl {
 cudaError_t launch_pair_round2(int blocks, int threads, size_t smem, cudaStream_t st, const nr::pr::Pair2* pairs,
                                const nr::pr::Deal& deal, const nr::Task* tasks, const nr::RestArgs& ra, const uint32_t* pool,
-                               const nr::ScoreW& k, int* counter, int stride, int4* out, uint32_t* state) {
+                               const nr::ScoreW& k, int* counter, int stride, int4* out, uint32_t* state,
+                               uint32_t* kept) {
     static std::mutex mu;
     static bool done = false;
     {
@@ -13,7 +14,7 @@ cudaError_t launch_pair_round2(int blocks, int threads, size_t smem, cudaStream_
         cudaError_t e = prepare(nr::pr::pair_round2_kernel, done);
         if (e != cudaSuccess) return e;
     }
-    nr::pr::pair_round2_kernel<<<blocks, threads, smem, st>>>(pairs, deal, tasks, ra, pool, k, counter, stride, out, state);
+    nr::pr::pair_round2_kernel<<<blocks, threads, smem, st>>>(pairs, deal, tasks, ra, pool, k, counter, stride, out, state, kept);
     return cudaGetLastError();
 }
 }  // namespace nrl

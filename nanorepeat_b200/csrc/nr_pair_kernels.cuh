@@ -65,7 +65,14 @@ struct Pair2 {         // round 2: two tasks of one region (same template); b < 
     int32_t a, b;
     int32_t mark_col;  // |left|: an alignment that starts at a column <= mark_col passes the span test (:373)
     int32_t state_off; // where the pair's DP state after column |left| - 2 is kept for round 3 (units of 32 words), -1: not kept
+    int32_t check_col; // single-stripe pairs: first column of the dominance exit's checks (Sweep::run); -1: no exit
+    int32_t period;    // lcm(16, |motif|): columns between two checks
+    int32_t pad[2];
 };
+
+// d_counters slots of a round-2 launch: cells the dominance exit skipped, per half (rows x columns, padding included),
+// and (rows of real reads) x columns x 32, both as 64-bit sums
+constexpr int kExitSlot = 24;
 
 struct Pair3 {         // round 3: two LadderTasks of one region, either may be absent (< 0)
     int32_t a, b;
@@ -158,6 +165,12 @@ struct Sweep {
     const u32* resume;             // kPF: state kept by round 2, [word * 32 + lane]
     u32* save;                     // kP2: where to keep the state after column save_col (null: nowhere)
     int save_col;
+    bool exits;                    // kP2 dominance exit: on for this pair (the kept cut follows the profile in shared memory)
+    int check_col, period;
+    int next_check;                // step of the next check (-1: none)
+    int exit_st;                   // step at which the exit ended the sweep (-1: swept to the end)
+    u32* kept_io;                  // global, this warp's slot: the kept cut's hup_prev, f1_out, f2_out and the period,
+                                   // [word * 32 + lane] (no room in registers or in shared memory at R = 16)
     // state
     u32 H[R], E1[R], E2[R];
     u32 hup_prev, h_out, f1_out, f2_out;
@@ -460,9 +473,14 @@ struct Sweep {
 #define NR_PAIR2_MULTI_UNROLL 4
 #endif
     static constexpr int kUnroll = MODE == kP2 ? (MULTI ? NR_PAIR2_MULTI_UNROLL : NR_PAIR2_UNROLL) : (MULTI ? 1 : NR_PAIR3_UNROLL);
-    template <bool TRACK, bool SPECIAL = false>
+    // EXIT (kP2 single stripes): the dominance exit's checks at trip boundaries, where every lane is at the same step
+    template <bool TRACK, bool SPECIAL = false, bool EXIT = false>
     __device__ __forceinline__ void fast_until(int& st, int end, u32 one, unsigned four) {
         for (; st + 16 <= end; st += 16) {       // st is a multiple of 16 here
+            if (EXIT && st == next_check) {
+                if (dominated_then_keep()) { exit_st = st; return; }
+                next_check += (int)__ldcg(kept_io + 96 + lane);
+            }
             refill();
 #pragma unroll 1
             for (int b = 0; b < 16; b += kUnroll) {
@@ -472,10 +490,32 @@ struct Sweep {
         }
     }
 
+    // kP2 dominance exit.  The cut between two steps is everything the rest of the sweep reads: H, E1, E2 of every
+    // lane's rows and what is in flight between the lanes (the diagonal hup_prev; h_out is H[R - 1]; f1_out, f2_out).
+    // Returns whether the cut is <= the kept one in every half of every word, then keeps the cut.  The 3R planes go
+    // behind the profile in shared memory (14 KB per warp at R = 16), the three in-flight words to kept_io.  The first
+    // check compares with zeros and fails: no half of a live word is ever 0 (the floor keeps them >= 13).
+    __device__ __forceinline__ bool dominated_then_keep() {
+        u32* g = kept_io + lane;
+        const u32 khp = __ldcg(g), kf1 = __ldcg(g + 32), kf2 = __ldcg(g + 64);
+        u32 acc = (__vmaxu2(hup_prev, khp) ^ khp) | (__vmaxu2(f1_out, kf1) ^ kf1) | (__vmaxu2(f2_out, kf2) ^ kf2);
+        __stcg(g, hup_prev); __stcg(g + 32, f1_out); __stcg(g + 64, f2_out);
+        u32* snap = reinterpret_cast<u32*>(const_cast<uint4*>(prof) + StripeCfg<R>::PROF_INT4);
+#pragma unroll
+        for (int r = 0; r < R; ++r) {
+            u32* k = snap + r * 32 + lane;
+            const u32 kh = k[0], ke1 = k[R * 32], ke2 = k[2 * R * 32];
+            acc |= (__vmaxu2(H[r], kh) ^ kh) | (__vmaxu2(E1[r], ke1) ^ ke1) | (__vmaxu2(E2[r], ke2) ^ ke2);
+            k[0] = H[r]; k[R * 32] = E1[r]; k[2 * R * 32] = E2[r];
+        }
+        return __all_sync(kFull, acc == 0);
+    }
+
     // zone_start_: kPF, first step (of this sweep) at which a lane can be at a junction column
     __device__ __forceinline__ void run(u32 one, unsigned four, int zone_start_) {
         init();
         zone_start = zone_start_;
+        exit_st = -1;
         const int n = t_len - col0;              // columns swept
         const int nsteps = n + 31;
         const int inside_end = ((n - 1) >> 4) << 4;     // steps 31 <= st < inside_end: every lane is inside the matrix
@@ -502,7 +542,24 @@ struct Sweep {
                 // those two checks unrolled four times measured slower here, unlike in the junction zone below)
                 slow_until(st, min(nsteps, ((mc + 32 + 15) >> 4) << 4), one, four);
             }
-            fast_until<true>(st, inside_end, one, four);
+            if (MULTI) {
+                fast_until<true>(st, inside_end, one, four);
+            } else {
+                // Dominance exit (DESIGN.md section 4.9).  Right of |left| the template repeats with period m and the
+                // DP is max-plus, so if the cut at step s is <= the cut at step s - P (P a multiple of m and of 16, both
+                // cuts wholly right of the last marked column) every later cell is <= one P columns to its left that
+                // was already folded into the record; only a strictly higher class replaces the record, so it is final.
+                // Checks every P steps from the trip at which lane 31 reaches check_col (and has passed mark_col).
+                next_check = -1;
+                if (exits && mc >= 0) {
+                    const int c0 = max(st, ((check_col - col0 + 32 + 15) >> 4) << 4);
+                    if (c0 + period < inside_end) next_check = c0;
+                    __stcg(kept_io + lane, 0u); __stcg(kept_io + 32 + lane, 0u); __stcg(kept_io + 64 + lane, 0u);
+                    __stcg(kept_io + 96 + lane, (u32)period);
+                }
+                fast_until<true, false, true>(st, inside_end, one, four);
+                if (exit_st >= 0) return;
+            }
         } else {
             // plain steps up to the first junction / marked column, then guard-free steps that look for both
             const int first = min(zone_start, mc >= 0 ? mc : zone_start);
@@ -582,7 +639,8 @@ __device__ __forceinline__ int next_item(const Deal& dl, bool& first, int* count
 // ---- round 2 -------------------------------------------------------------------------------------------------------
 template <int R>
 __device__ __forceinline__ void pair2_task(const Pair2& pt, const Task* __restrict__ tasks, const uint32_t* __restrict__ pool,
-                                           uint4* prof, int lane, u32 one, unsigned four, int4* out, u32* state) {
+                                           uint4* prof, int lane, u32 one, unsigned four, int4* out, u32* state,
+                                           unsigned long long* skipped, u32* kept) {
     const Task ta = tasks[pt.a];
     Task tb = ta;
     int q_b = 0;
@@ -596,7 +654,16 @@ __device__ __forceinline__ void pair2_task(const Pair2& pt, const Task* __restri
     sw.col0 = 0; sw.resume = nullptr;
     sw.save_col = pt.mark_col - 2;
     sw.save = (state && pt.state_off >= 0 && sw.save_col >= 0) ? state + (size_t)pt.state_off * 32 : nullptr;
+    sw.exits = pt.check_col >= 0;
+    sw.check_col = pt.check_col; sw.period = pt.period;
+    sw.kept_io = kept + (size_t)((blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5)) * 128);
     sw.run(one, four, 0);
+    if (sw.exit_st >= 0 && lane == 0) {
+        // lane l swept exit_st - l columns instead of t_len
+        const unsigned long long cols32 = 32ull * (unsigned)ta.t_len - (32ull * (unsigned)sw.exit_st - 496ull);
+        atomicAdd(&skipped[0], (unsigned long long)R * cols32);
+        atomicAdd(&skipped[1], (unsigned long long)(ta.q_len + q_b) * cols32);
+    }
     // per half: (score, smallest end column, mark of the best word there) -> one 32-bit key, warp maximum
 #pragma unroll
     for (int half = 0; half < 2; ++half) {
@@ -693,9 +760,9 @@ __device__ __forceinline__ void pair2_stripe_dispatch(int r, const Pair2& pt, in
 template <int R>
 __device__ __forceinline__ void pair2_dispatch(int r, const Pair2& pt, const Task* __restrict__ tasks,
                                                const uint32_t* __restrict__ pool, uint4* prof, int lane, u32 one,
-                                               unsigned four, int4* out, u32* state) {
-    if (r == R) { pair2_task<R>(pt, tasks, pool, prof, lane, one, four, out, state); return; }
-    if constexpr (R < kMaxRPair2) pair2_dispatch<R + 1>(r, pt, tasks, pool, prof, lane, one, four, out, state);
+                                               unsigned four, int4* out, u32* state, unsigned long long* skipped, u32* kept) {
+    if (r == R) { pair2_task<R>(pt, tasks, pool, prof, lane, one, four, out, state, skipped, kept); return; }
+    if constexpr (R < kMaxRPair2) pair2_dispatch<R + 1>(r, pt, tasks, pool, prof, lane, one, four, out, state, skipped, kept);
 }
 
 // Round 2: the batch's 32-bit entries (stripes of long reads first: they are the critical path) and then its pairs, one
@@ -704,7 +771,8 @@ __device__ __forceinline__ void pair2_dispatch(int r, const Pair2& pt, const Tas
 #ifdef NR_DEFINE_PAIR_ROUND2_KERNEL      // defined by the one translation unit that owns this kernel (nr_launch_pair2.cu)
 __global__ void __launch_bounds__(32 * kWarpsPerBlock, 1)
 pair_round2_kernel(const Pair2* __restrict__ pairs, Deal dl, const Task* __restrict__ tasks, RestArgs ra,
-                   const uint32_t* __restrict__ pool, ScoreW scw, int* counter, int smem_stride, int4* out, u32* state) {
+                   const uint32_t* __restrict__ pool, ScoreW scw, int* counter, int smem_stride, int4* out, u32* state,
+                   u32* kept) {
     extern __shared__ uint4 psmem[];
     const ScoreView<true> sc(scw);
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
@@ -727,7 +795,8 @@ pair_round2_kernel(const Pair2* __restrict__ pairs, Deal dl, const Task* __restr
         const Pair2 pt = pairs[i - ra.n_order];
         int q = tasks[pt.a].q_len;
         if (pt.b >= 0) q = max(q, tasks[pt.b].q_len);
-        pair2_dispatch<kMinR>(pair_rows(q), pt, tasks, pool, prof, lane, (u32)sc.one, sc.four, out, state);
+        pair2_dispatch<kMinR>(pair_rows(q), pt, tasks, pool, prof, lane, (u32)sc.one, sc.four, out, state,
+                              reinterpret_cast<unsigned long long*>(counter + kExitSlot), kept);
     }
 }
 #endif

@@ -35,7 +35,8 @@ class LaunchInfo(ctypes.Structure):
     _fields_ = [("paired_cells", ctypes.c_int64), ("rest_cells", ctypes.c_int64), ("n_pairs", ctypes.c_int32),
                 ("n_rest", ctypes.c_int32), ("n_redo", ctypes.c_int32), ("reserved", ctypes.c_int32),
                 ("paired_ms", ctypes.c_float), ("rest_ms", ctypes.c_float), ("redo_ms", ctypes.c_float),
-                ("reserved2", ctypes.c_float), ("paired_useful_cells", ctypes.c_int64), ("rest_useful_cells", ctypes.c_int64)]
+                ("reserved2", ctypes.c_float), ("paired_useful_cells", ctypes.c_int64), ("rest_useful_cells", ctypes.c_int64),
+                ("planned_paired_cells", ctypes.c_int64), ("planned_paired_useful_cells", ctypes.c_int64)]
 
     def as_dict(self):
         return {n: getattr(self, n) for n, _ in self._fields_ if not n.startswith("reserved")}
