@@ -259,6 +259,41 @@ int nr_estimate_regions(const nr_scoring_t* sc, int32_t fast_mode, int32_t n_reg
                         nr_stats_t* stats /* nullable: summed over the batches of the call */);
 
 /*
+ * Step 1 of any number of regions in ONE call: both anchors in every raw read and the core / middle positions
+ * (nanoRepeat_bam.py:165-234), what find_anchor_locations_in_reads does per region with minimap2 (:260-286).
+ * Per read the four exact alignments (left / right anchor x read / its reverse complement; the anchor is the query, the
+ * read strand the template); a hit is an alignment scoring >= min_dp_score; per anchor the hits sorted by score, '+'
+ * first on a tie; an anchor is good with one hit, or with two when AS0 > 1.5 * AS1 (:165-179); a read is accepted when
+ * both anchors are good and dist = right.qstart - left.qend (0 when the strands differ) > -10 (:195-211); the core is
+ * [left.qend - 100, right.qstart + 100) clamped to the read, the middle [left.qend, right.qstart) (:221-234), both in
+ * the orientation of the left anchor's strand.  Two kernel launches per call, whatever the number of regions.
+ * A read that is empty, longer than nr_limits' template limit or holds a character other than ACGTacgt is not scored
+ * (no hit; nr_stats_t.n_skipped counts the last two); an anchor may hold any character (N scores -ambiguous).
+ * Needs map-ont scoring with min_dp_score >= 10 * match (every preset): a hit then spans >= 10 read bases, so the
+ * reference's align_len < 10 test (:173) never decides.
+ */
+typedef struct nr_anchor_region_t {
+    const char* left;  int32_t n_left;      /* RepeatRegion.left_anchor_seq  */
+    const char* right; int32_t n_right;     /* RepeatRegion.right_anchor_seq */
+    int32_t n_reads;
+    const char* reads; int64_t reads_len;   /* the region's raw reads: n_reads lines separated by '\n' */
+} nr_anchor_region_t;
+typedef struct nr_anchor_read_t {           /* one per read, concatenated in region order */
+    uint8_t accepted;                       /* the read enters read_dict (both anchors good, dist > -10) */
+    uint8_t left_good, right_good;          /* left_anchor_is_good / right_anchor_is_good */
+    uint8_t strand;                         /* accepted reads: '+' or '-' (the left anchor's strand); else 0 */
+    uint8_t left_strand, right_strand;      /* strand of each anchor's best hit: '+', '-', 0 = no hit */
+    uint8_t pad[2];
+    int32_t read_len;
+    int32_t dist_between_anchors;           /* both anchors good: right.qstart - left.qend, or 0 across strands */
+    int32_t core_start, core_end, mid_start, mid_end, left_buffer, right_buffer;   /* accepted reads */
+    nr_aln_t left, right;                   /* best hit of each anchor as (AS, qstart, qend) on its strand; score 0: none;
+                                               qstart is recovered for good anchors only (-1 otherwise) */
+} nr_anchor_read_t;
+int nr_anchor_regions(const nr_scoring_t* sc, int32_t n_regions, const nr_anchor_region_t* regions, nr_anchor_read_t* out,
+                      nr_stats_t* stats /* nullable: algorithmic cells = sum of 2 * (|left| + |right|) * |read| */);
+
+/*
  * Joint path (nanoRepeat-joint: two neighbouring repeats quantified together).  The reference aligns every read against
  * a grid of templates left + motif1*k1 + mid + motif2*k2 + right with `minimap2 -c --eqx` (nanoRepeat_joint.py:315-343,
  * :397-419) and re-scores each alignment's CIGAR inside the window [|left| - 10, |left| + m1 k1 + |mid| + m2 k2 + 10)

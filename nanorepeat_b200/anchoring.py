@@ -1,6 +1,7 @@
 """Step 1 of the reference's per-region pipeline on the GPU: locate the two anchors in every read and cut the core.
 
-    find_anchor_locations_in_reads   <- reference src/NanoRepeat/nanoRepeat_bam.py:260-286 (+ :165-258)
+    find_anchor_locations_in_regions <- reference src/NanoRepeat/nanoRepeat_bam.py:260-286 (+ :165-258), many regions
+    find_anchor_locations_in_reads   <- the same for one region
     make_core_seq_fastq              <- reference src/NanoRepeat/nanoRepeat_bam.py:288-331
 
 The reference aligns every read of the region to `left_anchor` / `right_anchor` (<= 1000 bp each) with
@@ -17,8 +18,11 @@ rule: the candidate hits of an anchor are its best exact alignment on each stran
 "second AS" is the other strand's; `mapq > 30` is taken as true whenever the 1.5 x rule holds (mapq is a function of
 exactly that score ratio and chain properties this engine does not have); `align_len < 10` cannot occur above -s.
 A read longer than the engine's template limit (65 471 bases) is left out, as a read minimap2 printed nothing for.
+The rules run inside the library (nr_anchor_regions, include/nanorepeat_b200.h), one call for any number of regions.
 """
 import os
+
+import numpy as np
 
 from . import engine
 from .presets import get_preset_for_minimap2
@@ -55,94 +59,66 @@ class AnchorHit:
         self.mapq = 60
 
 
-def check_anchor_mapping(hits):
-    """nanoRepeat_bam.py:165-179 on hits sorted by align_score, best first."""
-    if len(hits) == 0:
-        return False
-    if len(hits) == 1:
-        return True
-    if hits[0].align_len < 10:
-        return False
-    return hits[0].align_score > 1.5 * hits[1].align_score and hits[0].mapq > 30
+def _reads_of(repeat_region, reads):
+    """(names, sequences) of a region's reads: given as such, as {name: sequence}, or (None) from its region FASTQ."""
+    if reads is None:
+        return read_fastq(repeat_region.region_fq_file)
+    if isinstance(reads, dict):
+        return list(reads), list(reads.values())
+    return reads
 
 
-def locate_anchors(data_type, left_anchor_seq, right_anchor_seq, read_seqs):
-    """-> per read (left hits, right hits), each a list of AnchorHit sorted by score, best first ('+' first on a tie)."""
+def find_anchor_locations_in_regions(data_type, repeat_regions, region_reads, read_class=None):
+    """Reference nanoRepeat_bam.py:260-286 + :181-234 for many regions in ONE library call (nr_anchor_regions: two
+    kernel launches however many regions): fills every region's read_dict with a Read per accepted read
+    (dist_between_anchors, strand, core / mid positions, buffer lengths, left_anchor_paf / right_anchor_paf).
+    region_reads: per region (names, sequences), {name: sequence} or None (the region's region_fq_file, which is what the
+    reference hands minimap2, :279).  read_class: the Read class to instantiate (default: this package's)."""
+    if len(repeat_regions) != len(region_reads):
+        raise ValueError("one read set per region")
     get_preset_for_minimap2(data_type)
     sc = engine.get_preset(data_type)
-    n = len(read_seqs)
-    if n == 0:
-        return []
-    rc = [rev_comp(s) for s in read_seqs]
-    anchors, targets = [], []
-    for fwd, rev in zip(read_seqs, rc):
-        anchors += [left_anchor_seq, left_anchor_seq, right_anchor_seq, right_anchor_seq]
-        targets += [fwd, rev, fwd, rev]
-    recs = engine.score_tasks(anchors, targets, sc)          # the anchor is the DP's query: (tstart, tend) are read coordinates
-    out = []
-    for r in range(n):
-        per_anchor = []
-        for a in range(2):
-            hits = []
-            for s, strand in enumerate("+-"):
-                rec = recs[4 * r + 2 * a + s]
-                if rec["score"] > 0 and rec["score"] >= sc.min_dp_score:
-                    hits.append(AnchorHit(strand, int(rec["score"]), int(rec["tstart"]), int(rec["tend"])))
-            hits.sort(key=lambda h: h.align_score, reverse=True)           # stable: '+' first on a tie (:190-191)
-            per_anchor.append(hits)
-        out.append(tuple(per_anchor))
-    return out
+    if read_class is None:
+        from .repeat_region import Read as read_class
+    named = [_reads_of(rr, reads) for rr, reads in zip(repeat_regions, region_reads)]
+    res, _stats = engine.anchor_regions(sc, [rr.left_anchor_seq for rr in repeat_regions],
+                                        [rr.right_anchor_seq for rr in repeat_regions], [list(seqs) for _names, seqs in named])
+    col = {k: res[k].tolist() for k in ("read_len", "dist_between_anchors", "core_start", "core_end", "mid_start", "mid_end",
+                                        "left_buffer", "right_buffer", "strand", "left_strand", "right_strand")}
+    for side in ("left", "right"):
+        for f in ("score", "tstart", "tend"):
+            col[side + f] = res[side][f].tolist()
+    accepted = np.flatnonzero(res["accepted"]).tolist()
+    first = 0
+    a = 0
+    for rr, (names, _seqs) in zip(repeat_regions, named):
+        end = first + len(names)
+        while a < len(accepted) and accepted[a] < end:
+            i = accepted[a]
+            a += 1
+            name = names[i - first]
+            read = read_class()
+            read.read_name = name
+            read.full_read_len = col["read_len"][i]
+            read.left_anchor_is_good = read.right_anchor_is_good = read.both_anchors_are_good = True
+            read.left_anchor_paf = AnchorHit(chr(col["left_strand"][i]), col["leftscore"][i], col["lefttstart"][i], col["lefttend"][i])
+            read.right_anchor_paf = AnchorHit(chr(col["right_strand"][i]), col["rightscore"][i], col["righttstart"][i],
+                                              col["righttend"][i])
+            read.dist_between_anchors = col["dist_between_anchors"][i]
+            rr.read_dict[name] = read
+            rr.buffer_len = BUFFER_LEN
+            read.core_seq_start_pos, read.core_seq_end_pos = col["core_start"][i], col["core_end"][i]
+            read.mid_seq_start_pos, read.mid_seq_end_pos = col["mid_start"][i], col["mid_end"][i]
+            read.left_buffer_len, read.right_buffer_len = col["left_buffer"][i], col["right_buffer"][i]
+            read.strand = chr(col["strand"][i])
+        first = end
+    return
 
 
 def find_anchor_locations_in_reads(data_type, repeat_region, num_cpu=1, reads=None, read_class=None):
-    """Reference nanoRepeat_bam.py:260-286 + :181-234: fills repeat_region.read_dict with a Read per accepted read
-    (dist_between_anchors, strand, core / mid positions, buffer lengths).
-    reads: (names, sequences) or {name: sequence}; default: repeat_region.region_fq_file, which is what the reference
-    hands minimap2 (:279).  read_class: the Read class to instantiate (default: this package's)."""
-    if reads is None:
-        names, seqs = read_fastq(repeat_region.region_fq_file)
-    elif isinstance(reads, dict):
-        names, seqs = list(reads), list(reads.values())
-    else:
-        names, seqs = reads
-    if read_class is None:
-        from .repeat_region import Read as read_class
-    hits = locate_anchors(data_type, repeat_region.left_anchor_seq, repeat_region.right_anchor_seq, seqs)
-    for name, seq, (left_hits, right_hits) in zip(names, seqs, hits):
-        if not left_hits and not right_hits:
-            continue                                                        # no PAF line for this read (:183)
-        read = read_class()
-        read.read_name = name
-        read.full_read_len = len(seq)
-        read.both_anchors_are_good = False
-        read.left_anchor_is_good = check_anchor_mapping(left_hits)         # :195-196
-        read.right_anchor_is_good = check_anchor_mapping(right_hits)
-        if not read.left_anchor_is_good or not read.right_anchor_is_good:
-            continue
-        left, right = left_hits[0], right_hits[0]
-        read.left_anchor_paf, read.right_anchor_paf = left, right
-        repeat_region_length = 0
-        if left.strand == right.strand:                                     # :206-207
-            repeat_region_length = right.qstart - left.qend
-        if repeat_region_length > -10:                                      # :209-211
-            read.both_anchors_are_good = True
-            read.dist_between_anchors = repeat_region_length
-        if not read.both_anchors_are_good:
-            continue
-        repeat_region.read_dict[name] = read
-        repeat_region.buffer_len = BUFFER_LEN
-        read.core_seq_start_pos = left.qend - BUFFER_LEN                    # :221-234
-        read.core_seq_end_pos = right.qstart + BUFFER_LEN
-        read.mid_seq_start_pos = left.qend
-        read.mid_seq_end_pos = right.qstart
-        if read.core_seq_start_pos < 0:
-            read.core_seq_start_pos = 0
-        if read.core_seq_end_pos > read.full_read_len:
-            read.core_seq_end_pos = read.full_read_len
-        read.left_buffer_len = left.qend - read.core_seq_start_pos
-        read.right_buffer_len = read.core_seq_end_pos - right.qstart
-        read.strand = "+" if left.strand == "+" else "-"
-    return
+    """Reference nanoRepeat_bam.py:260-286 + :181-234 for one region (find_anchor_locations_in_regions).
+    reads: (names, sequences) or {name: sequence}; default: repeat_region.region_fq_file."""
+    find_anchor_locations_in_regions(data_type, [repeat_region], [reads], read_class)
 
 
 def make_core_seq_fastq(repeat_region, reads=None, write_files=None):
@@ -150,12 +126,7 @@ def make_core_seq_fastq(repeat_region, reads=None, write_files=None):
     orientation, into repeat_region.read_core_seq_dict.  The two FASTQ files the reference also writes (the unmodified
     round1_and_round2_estimation reads core_sequences.fastq) are written when the region has a temp_out_dir, or on
     request; this package's own operators read the dictionary."""
-    if reads is None:
-        names, seqs = read_fastq(repeat_region.region_fq_file)
-    elif isinstance(reads, dict):
-        names, seqs = list(reads), list(reads.values())
-    else:
-        names, seqs = reads
+    names, seqs = _reads_of(repeat_region, reads)
     if write_files is None:
         write_files = bool(getattr(repeat_region, "temp_out_dir", None))
     core_f = mid_f = None

@@ -128,6 +128,7 @@ SYMBOLS = {
     "nr_batch_launch_info": (ctypes.c_int, [ctypes.c_void_p, ctypes.POINTER(LaunchInfo)]),
     "nr_batch_destroy": (None, [ctypes.c_void_p]),
     "nr_last_stats": (ctypes.c_int, [ctypes.POINTER(Stats)]),
+    "nr_anchor_regions": (ctypes.c_int, [_scp, ctypes.c_int32, ctypes.c_void_p, ctypes.c_void_p, ctypes.POINTER(Stats)]),
     "nr_window_tasks": (ctypes.c_int, [_scp, ctypes.c_int32, _cpp, _i32p, _cpp, _i32p, _i32p, _i32p, ctypes.c_void_p, ctypes.c_void_p]),
     "nr_joint_grid": (ctypes.c_int, [_scp, ctypes.c_char_p, ctypes.c_int32, ctypes.c_char_p, ctypes.c_int32, ctypes.c_char_p,
                                      ctypes.c_int32, ctypes.c_char_p, ctypes.c_int32, ctypes.c_char_p, ctypes.c_int32,
@@ -542,6 +543,54 @@ def estimate_regions(sc, fast_mode, lefts, rights, motifs, cores, dists, max_dis
                                      r3_state.ctypes.data, T.ctypes.data_as(_i32p), ctypes.byref(st)))
     del keep
     return dict(r1=r1, r2=r2, r2_valid=r2_valid.astype(bool), r3=r3, r3_state=r3_state, T=T[:n], stats=st.as_dict())
+
+
+# nr_anchor_region_t / nr_anchor_read_t as numpy records (same layout)
+ANCHOR_REGION_DTYPE = np.dtype([("left", "<u8"), ("n_left", "<i4"), ("right", "<u8"), ("n_right", "<i4"), ("n_reads", "<i4"),
+                                ("reads", "<u8"), ("reads_len", "<i8")], align=True)
+ANCHOR_READ_DTYPE = np.dtype([("accepted", "u1"), ("left_good", "u1"), ("right_good", "u1"), ("strand", "u1"),
+                              ("left_strand", "u1"), ("right_strand", "u1"), ("pad", "u1", (2,)), ("read_len", "<i4"),
+                              ("dist_between_anchors", "<i4"), ("core_start", "<i4"), ("core_end", "<i4"), ("mid_start", "<i4"),
+                              ("mid_end", "<i4"), ("left_buffer", "<i4"), ("right_buffer", "<i4"), ("left", ALN_DTYPE),
+                              ("right", ALN_DTYPE)], align=True)
+assert ANCHOR_REGION_DTYPE.itemsize == 48 and ANCHOR_READ_DTYPE.itemsize == 64
+
+
+def anchor_regions(sc, lefts, rights, reads):
+    """nr_anchor_regions: Step 1 (anchors, acceptance, core positions) of many regions in one call into the library.
+    lefts / rights: one str per region; reads: per region a list of str (raw reads, any strand).
+    -> (ANCHOR_READ_DTYPE array over all reads in region order, stats dict)."""
+    n = len(lefts)
+    if len(rights) != n or len(reads) != n:
+        raise ValueError("one left anchor, right anchor and read list per region")
+    n_reads = np.fromiter(map(len, reads), np.int64, n)
+    flat = list(itertools.chain.from_iterable(reads))
+    # a read that holds a newline (or any other character than ACGT) is not scored: it travels as one of N, never as
+    # two lines
+    flat = [r.replace("\n", "N") if "\n" in r else r for r in flat]
+    tab = np.zeros(max(n, 1), ANCHOR_REGION_DTYPE)
+    keep = []
+    for name, seqs in (("left", lefts), ("right", rights)):
+        big, ptr, off = _joined([s.encode("ascii", "replace").decode() for s in seqs])
+        keep.append(big)
+        tab[name][:n] = ptr + off[:-1]
+        tab["n_" + name][:n] = off[1:] - off[:-1]
+    big = "\n".join(flat).encode("ascii", "replace")          # a non-ASCII character becomes '?': the read is not scored
+    keep.append(big)
+    base = ctypes.cast(ctypes.c_char_p(big), ctypes.c_void_p).value or 0
+    clen = np.fromiter(map(len, flat), np.int64, len(flat))
+    csum = np.zeros(len(flat) + 1, np.int64)
+    np.cumsum(clen + 1, out=csum[1:])                          # start of every line
+    first = np.zeros(n + 1, np.int64)
+    np.cumsum(n_reads, out=first[1:])
+    tab["reads"][:n] = base + csum[first[:-1]]
+    tab["reads_len"][:n] = np.maximum(csum[first[1:]] - csum[first[:-1]] - 1, 0)
+    tab["n_reads"][:n] = n_reads
+    out = np.zeros(max(len(flat), 1), ANCHOR_READ_DTYPE)
+    st = Stats()
+    _check(lib().nr_anchor_regions(ctypes.byref(sc), n, tab.ctypes.data, out.ctypes.data, ctypes.byref(st)))
+    del keep
+    return out[:len(flat)], st.as_dict()
 
 
 WINDOW_DTYPE = np.dtype([("score", "<i4"), ("window_score", "<i4")])

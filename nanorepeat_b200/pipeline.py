@@ -25,8 +25,8 @@ def quantify_regions(repeat_regions, region_reads, data_type="ont", fast_mode=Fa
     reference would not phase it) and `num_removed_reads`."""
     if len(repeat_regions) != len(region_reads):
         raise ValueError("one read set per region")
+    anchoring.find_anchor_locations_in_regions(data_type, repeat_regions, region_reads)   # Step 1 (:669-672), one call
     for rr, reads in zip(repeat_regions, region_reads):
-        anchoring.find_anchor_locations_in_reads(data_type, rr, 1, reads=reads)      # Step 1 (:669-672)
         anchoring.make_core_seq_fastq(rr, reads=reads, write_files=False)
     estimate_regions(repeat_regions, data_type, fast_mode)                            # Steps 2 and 3 (:675-679), batched
     if phase:                                                                          # Step 4 (:684), batched
