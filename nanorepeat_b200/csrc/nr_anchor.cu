@@ -13,6 +13,7 @@
 //      tie-break.  The library checks score and end and fails the call rather than return another start.
 //      Anchors too long for a 16-bit half are scored here too, against whole strands.
 // Then the reference's rules, on the host.
+#include "nr_batch.h"
 #include "nr_internal.h"
 #include "nr_launch_anchor.h"
 
@@ -35,7 +36,6 @@ namespace {
         }                                                                                                \
     } while (0)
 
-constexpr int kMaxTlen = 65535 - 64;               // the packed kernels' template limit (nr_limits)
 constexpr int kMaxPairAnchor = (65535 - 65) / 4;   // a half holds 2 * score + 65 and score <= 2 * |anchor| (map-ont)
 constexpr int kBufferLen = 100;                    // nanoRepeat_bam.py:221
 
@@ -72,23 +72,6 @@ void pair_shape(int rows, int& R, int& S) {
 
 struct Cand { int score = 0, tstart = -1, tend = 0; };      // one anchor on one strand of one read
 
-// 2-bit pool of the call: anchors are queries (an ambiguity plane for bases other than ACGT), read strands templates
-struct SeqPool {
-    std::vector<uint32_t> words;
-    long long add(const char* s, int len, bool is_query) {
-        const size_t w0 = words.size();
-        words.resize(w0 + (size_t)(len + 15) / 16 + 1, 0u);
-        if (!nri::pack(s, len, words.data() + w0)) {
-            if (!is_query) { words.resize(w0); return -1; }
-            const size_t at = words.size();
-            words.resize(at + (size_t)(len + 31) / 32, 0u);
-            nri::ambiguity(s, len, words.data() + at);
-            words[w0 + (size_t)(len + 15) / 16] = (uint32_t)(at - w0);
-        }
-        return (long long)w0;
-    }
-};
-
 int anchor_regions(const nr_scoring_t* sc, int n_regions, const nr_anchor_region_t* regs, nr_anchor_read_t* out, nr_stats_t* stats) {
     // ---- reads of every region: split the lines, pack both strands ----
     std::vector<long long> first(n_regions + 1, 0);
@@ -121,7 +104,7 @@ int anchor_regions(const nr_scoring_t* sc, int n_regions, const nr_anchor_region
     int rc = nri::ensure_init();
     if (rc) return rc;
     nr_stats_t st = {};
-    SeqPool pool;
+    nrh::Pool pool;        // anchors are queries (an ambiguity plane for bases other than ACGT), read strands templates
     {
         size_t words = 0;
         for (long long i = 0; i < total; ++i) words += 2 * ((size_t)(rlen[i] + 15) / 16 + 1);
@@ -137,7 +120,7 @@ int anchor_regions(const nr_scoring_t* sc, int n_regions, const nr_anchor_region
     std::vector<std::string> rev(total);
     for (long long i = 0; i < total; ++i) {
         if (rlen[i] == 0) continue;
-        if (rlen[i] > kMaxTlen) { ++st.n_skipped; continue; }
+        if (rlen[i] > nrh::kMaxTlen) { ++st.n_skipped; continue; }
         const long long w = pool.add(rptr[i], rlen[i], false);
         if (w < 0) { ++st.n_skipped; continue; }
         fwd_word[i] = w;
@@ -352,8 +335,7 @@ extern "C" int nr_anchor_regions(const nr_scoring_t* sc, int32_t n_regions, cons
                                  nr_stats_t* stats) {
     if (nri::check(sc)) return nri::last_code();
     if (n_regions < 0 || (n_regions > 0 && !regions)) return nri::fail_msg(NR_ERR_ARG, "nr_anchor_regions: bad arguments");
-    if (!(sc->match == 2 && sc->mismatch == 4 && sc->gap_open1 == 4 && sc->gap_ext1 == 2 && sc->gap_open2 == 24 &&
-          sc->gap_ext2 == 1 && sc->ambiguous == 1) || sc->min_dp_score < 10 * sc->match)
+    if (!nrh::is_map_ont(*sc) || sc->min_dp_score < 10 * sc->match)
         return nri::fail_msg(NR_ERR_ARG, "nr_anchor_regions: needs map-ont scoring with min_dp_score >= 10 * match");
     long long total = 0;
     for (int g = 0; g < n_regions; ++g) total += std::max(0, regions[g].n_reads);

@@ -6,21 +6,17 @@
 // construction over any number of regions, cost sorting, launches of the sm_100a kernels in nr_kernels.cuh, result
 // gather and the round-3 selection of nanoRepeat_bam.py:423-431.
 // There is no CPU compute fallback: without a CUDA device every compute call fails with NR_ERR_CUDA.
-#include "../../include/nanorepeat_b200.h"
-#include "nr_launch.h"
+#include "nr_batch.h"
 
 #include <algorithm>
-#include <numeric>
 #if defined(__x86_64__)
 #include <tmmintrin.h>
 #endif
 #include <atomic>
-#include <chrono>
 #include <cstdarg>
 #include <cstdio>
 #include <cstdlib>
 #include <cstring>
-#include <functional>
 #include <mutex>
 #include <new>
 #include <string>
@@ -29,13 +25,17 @@
 #include <unordered_map>
 #include <vector>
 
+using namespace nrh;
+
 namespace {
 
 thread_local std::string g_err;
 thread_local int g_code = 0;
 thread_local nr_stats_t g_last_stats = {};
 
-int fail(int code, const char* fmt, ...) {
+}  // namespace
+
+int nrh::fail(int code, const char* fmt, ...) {
     char buf[512];
     va_list ap;
     va_start(ap, fmt);
@@ -46,6 +46,8 @@ int fail(int code, const char* fmt, ...) {
     return code;
 }
 
+namespace {
+
 #define CUDA_TRY(expr)                                                                          \
     do {                                                                                        \
         cudaError_t e__ = (expr);                                                               \
@@ -54,8 +56,6 @@ int fail(int code, const char* fmt, ...) {
                         __FILE__, __LINE__);                                                    \
     } while (0)
 
-constexpr int kMaxScore = 32767;   // signed 16-bit score field of the packed DP word
-constexpr int kMaxTlen = 65535 - 64; // unsigned 16-bit span field, minus the wavefront skew (step counters share it)
 using nr::kWarpsPerBlock;
 
 // ---- context + caching allocator -----------------------------------------------------------------------------
@@ -229,6 +229,12 @@ bool pack_seq(const char* s, int len, uint32_t* w) {
     return bad == 0;
 }
 
+// Bit plane of the bases of s that are not ACGT (bit i & 31 of word i >> 5); m holds (len + 31) / 32 zeroed words.
+void ambiguity_plane(const char* s, int len, uint32_t* m) {
+    for (int i = 0; i < len; ++i)
+        if (g_bad.t[(unsigned char)s[i]]) m[i >> 5] |= 1u << (i & 31);
+}
+
 // fn(i) for i in [0, n) on a few host threads (packing thousands of reads is the host's largest cost per call)
 template <class F>
 void parallel_for(int n, int grain, F fn) {
@@ -245,138 +251,6 @@ void parallel_for(int n, int grain, F fn) {
     for (auto& x : th) x.join();
 }
 
-// Bit plane of the bases of s that are not ACGT (bit i & 31 of word i >> 5); m holds (len + 31) / 32 zeroed words.
-void ambiguity_plane(const char* s, int len, uint32_t* m) {
-    for (int i = 0; i < len; ++i)
-        if (g_bad.t[(unsigned char)s[i]]) m[i >> 5] |= 1u << (i & 31);
-}
-
-// Sequence pool.  Every sequence starts on a word boundary and is followed by one slack word (kernels prefetch one word
-// ahead).  For a READ the slack word doubles as the link to its ambiguity plane: 0 = ACGT only, otherwise the plane
-// starts that many words behind the read's first word (nr_kernels.cuh, read_has_ambiguous).  Templates must be ACGT.
-struct Pool {
-    std::vector<uint32_t> words;
-    // append; returns first word index, or -1 on a non-ACGT character (ambiguous_ok: append the plane instead)
-    long long add(const char* s, int len, bool ambiguous_ok = false) {
-        const size_t w0 = words.size();
-        const size_t nw = (size_t)(len + 15) / 16 + 1;
-        words.resize(w0 + nw, 0u);
-        if (!pack_seq(s, len, words.data() + w0)) {
-            if (!ambiguous_ok) { words.resize(w0); return -1; }
-            link_plane(w0, s, len);
-        }
-        return (long long)w0;
-    }
-    // append the ambiguity plane of the read packed at word w0 and link it from the read's slack word
-    void link_plane(size_t w0, const char* s, int len) {
-        const size_t at = words.size();
-        words.resize(at + (size_t)(len + 31) / 32, 0u);
-        ambiguity_plane(s, len, words.data() + at);
-        words[w0 + (size_t)(len + 15) / 16] = (uint32_t)(at - w0);
-    }
-};
-
-struct Launch {      // one persistent launch per batch
-    bool ladder;     // ladder_kernel over nr_batch::ltasks instead of exact_kernel over nr_batch::tasks
-    int R;           // tallest stripe of the launch: sizes the shared memory per warp
-    int count;
-    int blocks;
-    bool fixed;      // scoring == map-ont: kernels with immediate constants
-    // paired launch (nr_pair_kernels.cuh): two reads of one region per warp
-    int n_pairs;
-    int pair_R;
-    int pair_blocks;
-    int redo_R;                 // tallest stripe among the paired round-3 reads: sizes the redo launch
-};
-
-struct RegionInfo {   // one add_round2 / add_round3 call
-    int n_left = 0, n_right = 0, motif_len = 0;
-    int first_read = 0, n_reads = 0;
-    std::string left, motif;      // round 2 keeps them for a round-3 batch built over the same reads
-};
-
-}  // namespace
-
-enum BatchKind { KIND_TASKS = 0, KIND_ROUND2 = NR_KIND_ROUND2, KIND_ROUND3 = NR_KIND_ROUND3 };
-
-struct nr_batch {
-    BatchKind kind = KIND_TASKS;
-    nr_scoring_t sc = {};
-    bool committed = false;
-    std::vector<nr::Task> tasks;
-    std::vector<nr::LadderTask> ltasks;       // round 3 in ladder mode (tasks stays empty)
-    std::vector<nr::LadderRegion> lregs;
-    bool ladder = false;
-    bool flag = false;                        // ladder on flag words: d_out holds (score, spans both, ends in right)
-    bool pair = false;                        // paired u16x2 kernels where a task is eligible (round 2: flags kind; round 3: mode 3)
-    bool r2flags = false;                     // round 2: records are (score, span predicate, tend); no tstart
-    std::vector<nr::pr::Pair2> pairs2;        // single-stripe pairs first (n_pairs2_single), then the pairs of long reads
-    std::vector<nr::pr::Pair3> pairs3;
-    int n_pairs2_single = 0, n_pairs3_single = 0;
-    bool long_redone = false;                 // the host-side rescoring of this run's undecidable long reads is merged
-    int n_long_pairs = 0;                     // pairs of long reads: their stripes are entries of order[] (nr::pr::kPairEntry)
-    void* d_pairs = nullptr;                  // inside the blob
-    uint2* d_prung = nullptr;                 // round 3 pairs: (P, J) tokens per rung of a pair's ladder
-    size_t prung_bytes = 0;
-    int32_t* d_redo = nullptr;                // round 3 pairs: reads to rescore on 32-bit flag words
-    size_t redo_bytes = 0;
-    cudaEvent_t ev_t[6] = {};                 // nr_set_timing(1): start / end of the 32-bit, paired and redo launches
-    bool timed[3] = {};
-    int* h_redo_count = nullptr;              // pinned
-    int* h_spin = nullptr;                    // pinned: the kernels' give-up flag after the run (long reads only)
-    long long paired_cells = 0, rest_cells = 0;
-    long long paired_useful = 0, rest_useful = 0;   // the same without padding: rows of real reads only
-    bool round2_exit = false;                 // the single-stripe round-2 pairs may end their sweeps early (Pair2::check_col)
-    size_t n_out = 0;                         // records in d_out / h_out
-    std::vector<int32_t> order;               // entries of the 32-bit launch: (task << 7) | code (nr_kernels.cuh)
-    std::vector<nr::CoopInfo> coop;           // scratch of the multi-stripe tasks
-    std::vector<int32_t> coop_idx;            // exact tasks: index into coop, -1 for single-stripe tasks
-    nr::CoopInfo* d_coop = nullptr;
-    int32_t* d_coop_idx = nullptr;
-    std::vector<int32_t> lt_src;              // round 3 over a round-2 batch's reads: that batch's task of every ladder task
-    uint32_t* d_state = nullptr;              // round 2 pairs: DP state after column |left| - 2, kept for round 3
-    uint32_t* d_kept = nullptr;               // round 2 dominance exit: 128 words per warp of the launch
-    size_t state_bytes = 0;
-    int* d_flags = nullptr;                   // progress flags of the multi-stripe tasks, zeroed before every run
-    size_t flags_bytes = 0;
-    Launch launch = {};
-    Pool pool;
-    // per-read bookkeeping (rounds 2 and 3)
-    std::vector<RegionInfo> regions;
-    int n_reads = 0;
-    int n_skipped = 0;                        // tasks / reads left unscored (template not ACGT, beyond the packed range)
-    int n_ambiguous_reads = 0;                // reads with a base other than ACGT (scored through an ambiguity plane)
-    std::vector<int32_t> read_region;
-    std::vector<int32_t> kmin, kmax;
-    std::vector<int64_t> rung_off;            // n_reads + 1 (round 3)
-    // device
-    void* d_blob = nullptr;                   // tasks | regions | order | pool | counters: one allocation, one H2D copy
-    size_t blob_bytes = 0;
-    void* h_blob = nullptr;                   // pinned staging of the same layout
-    nr::Task* d_tasks = nullptr;
-    nr::LadderTask* d_ltasks = nullptr;
-    nr::LadderRegion* d_lregs = nullptr;
-    int32_t* d_order = nullptr;
-    uint32_t* d_pool = nullptr;
-    int* d_counters = nullptr;
-    int4* d_out = nullptr;
-    size_t out_bytes = 0;
-    int4* d_scratch = nullptr;
-    size_t scratch_bytes = 0;
-    int4* h_out = nullptr;                    // pinned
-    int4* d_sel = nullptr;                    // flag ladder: per read (top score, n tied, sum k lo, sum k hi)
-    int4* h_sel = nullptr;                    // pinned
-    size_t sel_bytes = 0;
-    nr_stats_t stats = {};
-    bool ran = false;
-    cudaStream_t run_stream = nullptr;        // stream of the last nr_batch_run: fetch orders itself behind it
-    cudaEvent_t ev_uploaded = nullptr;        // recorded behind the upload on the library's stream
-    cudaEvent_t ev_done = nullptr;            // recorded behind the kernel and the result copy of nr_batch_run
-    int refs = 1;                             // the owner + round-3 batches that read this batch's packed reads
-    nr_batch* qsrc = nullptr;                 // round 3: the committed round-2 batch whose reads are reused
-};
-
-namespace {
 
 // shared memory per warp, in int4: query profile (+ backward junction vectors for the ladder kernel)
 int exact_smem_int4(int R) { return 4 * ((R + 3) / 4) * 32; }
@@ -419,505 +293,25 @@ nr::ScoreW score_words(const nr_scoring_t& sc) {
     return k;
 }
 
-size_t align_up(size_t x, size_t a) { return (x + a - 1) / a * a; }
-
-// NR_TRACE=1: host-side phase times of plan_batch on stderr (where a commit's half millisecond goes)
-struct PhaseTrace {
-    const bool on = getenv("NR_TRACE") != nullptr;
-    std::chrono::steady_clock::time_point t0 = std::chrono::steady_clock::now();
-    void mark(const char* what) {
-        if (!on) return;
-        const auto t1 = std::chrono::steady_clock::now();
-        fprintf(stderr, "[nr trace] %-28s %8.1f us   (ends at %10.1f us, thread %04x)\n", what,
-                std::chrono::duration<double, std::micro>(t1 - t0).count(), std::fmod(std::chrono::duration<double, std::micro>(t1.time_since_epoch()).count(), 1e8),
-                (unsigned)(std::hash<std::thread::id>()(std::this_thread::get_id()) & 0xffff));
-        t0 = t1;
-    }
-};
-
-bool is_map_ont(const nr_scoring_t& c) {
-    return c.match == 2 && c.mismatch == 4 && c.gap_open1 == 4 && c.gap_ext1 == 2 && c.gap_open2 == 24 && c.gap_ext2 == 1 &&
-           c.ambiguous == 1;
-}
-
-// Round 2's dominance exit (nr_pair_kernels.cuh, Sweep::run; DESIGN.md section 4.9).  NR_ROUND2_EXIT=0 turns it off
-// for the batches committed while it is set (A/B measurements); it changes no result either way.
-bool round2_exit_enabled() {
-    const char* e = getenv("NR_ROUND2_EXIT");
-    return !(e && atoi(e) == 0);
-}
-// A core is 100 read bases of left flank + repeat + 100 of right flank (nanoRepeat_bam.py:308-316), so its repeat
-// ends near column |left| + q - 100 of the template and the DP past it turns periodic within a few motif copies.  On
-// config 2 (tools/round2_exit_census.py) the sweep ends at |left| + q - 83 on average; checks from |left| + q - 192 find
-// the same exits as checks from |left| on (18.1 % of the region's cells), from |left| + q - 100 they find 16.5 %.
-int round2_check_col(int n_left, int q_len) { return std::max(n_left + 1, n_left + q_len - 192); }
-int round2_predicted_exit(int n_left, int q_len) { return n_left + std::max(q_len - 64, 32); }
-
-// Pair up the eligible tasks of one region (ids[]: task indices, all of the same template): neighbours in read length
-// share a warp, one per 16-bit half of the DP words (nr_pair_kernels.cuh).  key(i) orders the tasks.
-template <class Key, class Emit>
-void make_pairs(std::vector<int>& ids, Key key, Emit emit) {
-    // decreasing key, then increasing id: one 64-bit word per task, (key << 32) | ~id, sorted downwards
-    std::vector<uint64_t> w(ids.size());
-    for (size_t i = 0; i < ids.size(); ++i) w[i] = ((uint64_t)(uint32_t)key(ids[i]) << 32) | (uint32_t)~(uint32_t)ids[i];
-    std::sort(w.begin(), w.end(), std::greater<uint64_t>());
-    for (size_t i = 0; i < w.size(); ++i) ids[i] = (int)~(uint32_t)w[i];
-    for (size_t i = 0; i < ids.size(); i += 2) emit(ids[i], i + 1 < ids.size() ? ids[i + 1] : -1);
-}
-
-// Pair the eligible tasks, sort the rest (single-stripe | multi-stripe groups, each by decreasing cost), size the
-// launches, upload.
-int plan_batch(nr_batch* b) {
-    const bool ladder = b->ladder;
-    const int n = ladder ? (int)b->ltasks.size() : (int)b->tasks.size();
-    if (b->kind != KIND_ROUND3) b->n_out = b->tasks.size();
-    b->stats = {};
-    b->stats.n_tasks = (int64_t)b->n_out;
-    std::vector<long long> cost(n, 0);
-    std::vector<int> task_R(n, nr::kMinR), task_ns(n, 1), task_sweep(n, 0), task_rungs(n, 0);
-    // 1: runs on the paired kernels; 2: not scored -- an empty sequence, a template that is not ACGT (t_len < 0), or a
-    // task beyond the packed score / coordinate range: its record stays zero, which every caller reads as "the aligner
-    // printed nothing" (nanoRepeat_bam.py:421, :433); the rest of the batch is unaffected
-    std::vector<char> paired(n, 0);
-    const int max_r = ladder ? nr::kMaxRLadder : nr::kMaxRExact;
-    const bool fixed = is_map_ont(b->sc);
+// Allocates the buffers plan_batch sized, stages the blob's sections in pinned memory and uploads them on the library's
+// stream (asynchronously: nr_batch_run orders itself behind ev_uploaded).
+int upload_batch(nr_batch* b) {
     PhaseTrace trace;
-    for (int i = 0; i < n; ++i) {
-        int q_len, t_len, t_sweep;
-        if (ladder) {
-            const nr::LadderTask& t = b->ltasks[i];
-            const nr::LadderRegion& g = b->lregs[t.region];
-            const int flank = g.n_left + g.n_right;
-            q_len = t.q_len;
-            t_len = flank + g.m * t.kmax;                 // longest rung = columns swept (|R| backward, rest forward)
-            t_sweep = std::max(g.n_left + g.m * t.kmax, g.n_right);
-            const int rungs = t.kmax - t.kmin + 1;
-            task_rungs[i] = rungs;
-            b->stats.algorithmic_cells +=
-                (long long)q_len * ((long long)rungs * flank + (long long)g.m * (t.kmin + t.kmax) * rungs / 2);
-        } else {
-            const nr::Task& t = b->tasks[i];
-            q_len = t.q_len;
-            t_len = t_sweep = t.t_len;
-            if (t_len > 0) b->stats.algorithmic_cells += (long long)q_len * t_len;
-        }
-        if (q_len <= 0 || t_len <= 0) {
-            paired[i] = 2;
-            if (t_len < 0) ++b->n_skipped;
-            continue;
-        }
-        long long m = (long long)b->sc.match * std::min(q_len, t_len);
-        if (m > kMaxScore || t_len > kMaxTlen) {        // (its cells stay in the count of what was asked for)
-            paired[i] = 2;
-            ++b->n_skipped;
-            continue;
-        }
-        nr::stripe_shape(q_len, max_r, task_R[i], task_ns[i]);
-        task_sweep[i] = t_sweep;
-        cost[i] = (long long)task_ns[i] * 32 * task_R[i] * t_len;
-    }
-    trace.mark("task shapes");
-    // ---- paired launch: two reads of one region per warp ----
-    std::vector<long long> pair_cost;
-    std::vector<long long> deal_cost;     // round 2: the cost the pairs are dealt by, the sweep up to the predicted exit
-    Launch& L = b->launch;
-    L = {};
-    long long state_off = 0;
-    long long rung_off = 0;           // (P, J) token pairs of the paired ladders, single-stripe pairs first
-    if (b->pair && fixed && !ladder && b->kind == KIND_ROUND2) {
-        const bool exits = round2_exit_enabled();
-        for (const RegionInfo& g : b->regions) {
-            std::vector<int> ids;
-            for (int r = g.first_read; r < g.first_read + g.n_reads; ++r) {
-                const nr::Task& t = b->tasks[r];
-                if (!paired[r] && t.q_len >= 1 && t.q_len <= 32 * nr::pr::kMaxRPair2 && t.t_len >= 1) ids.push_back(r);
-            }
-            make_pairs(ids, [&](int i) { return b->tasks[i].q_len; }, [&](int x, int y) {
-                const int R = nr::pr::pair_rows(b->tasks[x].q_len);      // x is the longer read
-                nr::pr::Pair2 p = {x, y, g.n_left, -1, -1, 0, {0, 0}};
-                const int t_len = b->tasks[x].t_len;
-                int cols = t_len;
-                if (exits) {
-                    p.check_col = round2_check_col(g.n_left, b->tasks[x].q_len);
-                    p.period = 16 / std::gcd(16, g.motif_len) * g.motif_len;
-                    cols = std::min(t_len, round2_predicted_exit(g.n_left, b->tasks[x].q_len));
-                    b->round2_exit = true;
-                }
-                if (g.n_left >= 2 && state_off + nr::pr::state_words(R) < 0x7fffffffLL) {
-                    p.state_off = (int32_t)state_off;                    // round 3 resumes from here (nr_batch_begin_round3_from)
-                    state_off += nr::pr::state_words(R);
-                }
-                b->pairs2.push_back(p);
-                paired[x] = 1;
-                if (y >= 0) paired[y] = 1;
-                L.pair_R = std::max(L.pair_R, R);
-                pair_cost.push_back((long long)32 * R * t_len);
-                deal_cost.push_back((long long)32 * R * cols);
-                b->paired_useful += (long long)(b->tasks[x].q_len + (y >= 0 ? b->tasks[y].q_len : 0)) * t_len;
-            });
-        }
-    } else if (b->pair && fixed && ladder && b->flag) {
-        if (b->qsrc && !b->qsrc->pairs2.empty() && (int)b->lt_src.size() == n) {
-            // the reads were paired in round 2: same pairs, same halves, same rows per lane, so that the forward sweep
-            // can take over the DP state round 2 kept after column |left| - 2 instead of sweeping the left anchor again
-            const nr_batch* src = b->qsrc;
-            std::vector<int> src2lt(src->tasks.size(), -1);
-            for (int i = 0; i < n; ++i)
-                if (b->lt_src[i] >= 0) src2lt[b->lt_src[i]] = i;
-            for (int pi = 0; pi < src->n_pairs2_single; ++pi) {
-                const nr::pr::Pair2& p2 = src->pairs2[pi];
-                int la = src2lt[p2.a], lb = p2.b >= 0 ? src2lt[p2.b] : -1;
-                if (la >= 0 && paired[la]) la = -1;        // (not scored: beyond the packed range)
-                if (lb >= 0 && paired[lb]) lb = -1;
-                if (la < 0 && lb < 0) continue;
-                const nr::LadderRegion& g = b->lregs[b->ltasks[la >= 0 ? la : lb].region];
-                if (g.n_left <= 0 || g.n_right <= 0) continue;
-                const int q = std::max(src->tasks[p2.a].q_len, p2.b >= 0 ? src->tasks[p2.b].q_len : 0);
-                const int R = nr::pr::pair_rows(q);
-                int kmin = INT32_MAX, kmax = -1;
-                for (int t : {la, lb})
-                    if (t >= 0) { kmin = std::min(kmin, b->ltasks[t].kmin); kmax = std::max(kmax, b->ltasks[t].kmax); }
-                nr::pr::Pair3 p = {la, lb, (int32_t)rung_off, -1, R, {0, 0, 0}};
-                if (p2.state_off >= 0 && src->d_state && g.n_left >= 2 && g.n_left == p2.mark_col) p.state_off = p2.state_off;
-                rung_off += kmax - kmin + 1;
-                b->pairs3.push_back(p);
-                if (la >= 0) paired[la] = 1;
-                if (lb >= 0) paired[lb] = 1;
-                L.pair_R = std::max(L.pair_R, R);
-                const long long cols = (long long)g.n_right + g.n_left + (long long)g.m * kmax - (p.state_off >= 0 ? g.n_left - 1 : 0);
-                pair_cost.push_back((long long)32 * R * cols);
-                b->paired_useful += (long long)((la >= 0 ? b->ltasks[la].q_len : 0) + (lb >= 0 ? b->ltasks[lb].q_len : 0)) * cols;
-            }
-        }
-        for (int i0 = 0; i0 < n;) {
-            int i1 = i0;
-            while (i1 < n && b->ltasks[i1].region == b->ltasks[i0].region) ++i1;
-            const nr::LadderRegion& g = b->lregs[b->ltasks[i0].region];
-            std::vector<int> ids;
-            if (g.n_left > 0 && g.n_right > 0)
-                for (int i = i0; i < i1; ++i)
-                    if (!paired[i] && b->ltasks[i].q_len >= 1 && b->ltasks[i].q_len <= 32 * nr::pr::kMaxRPair3) ids.push_back(i);
-            make_pairs(ids, [&](int i) { return ((long long)b->ltasks[i].q_len << 20) + b->ltasks[i].kmax; }, [&](int x, int y) {
-                const nr::LadderTask& tx = b->ltasks[x];
-                int kmin = tx.kmin, kmax = tx.kmax;
-                if (y >= 0) { kmin = std::min(kmin, b->ltasks[y].kmin); kmax = std::max(kmax, b->ltasks[y].kmax); }
-                nr::pr::Pair3 p = {x, y, (int32_t)rung_off, -1, 0, {0, 0, 0}};
-                rung_off += kmax - kmin + 1;
-                b->pairs3.push_back(p);
-                paired[x] = 1;
-                if (y >= 0) paired[y] = 1;
-                const int R = nr::pr::pair_rows(tx.q_len);
-                L.pair_R = std::max(L.pair_R, R);
-                pair_cost.push_back((long long)32 * R * (g.n_right + g.n_left + (long long)g.m * kmax));
-                b->paired_useful += (long long)(tx.q_len + (y >= 0 ? b->ltasks[y].q_len : 0)) * (g.n_right + g.n_left + (long long)g.m * kmax);
-            });
-            i0 = i1;
-        }
-        if (rung_off > 0x7fffffffLL) return fail(NR_ERR_TOO_LARGE, "more than 2^31 rungs in one batch");
-        L.redo_R = L.pair_R;
-    }
-    trace.mark("pairing");
-    b->state_bytes = sizeof(uint32_t) * 32 * (size_t)state_off;
-    L.n_pairs = (int)pair_cost.size();
-    if (L.n_pairs) {            // pairs in decreasing cost: the tail of the persistent launch is made of the cheap ones
-        std::vector<int> po(L.n_pairs);
-        {
-            std::vector<uint64_t> w(L.n_pairs);      // (cost << 24) | ~index: pair costs stay below 2^40, pairs below 2^24
-            const std::vector<long long>& dc = deal_cost.empty() ? pair_cost : deal_cost;
-            for (int i = 0; i < L.n_pairs; ++i) w[i] = ((uint64_t)dc[i] << 24) | (uint32_t)(0xffffff - i);
-            std::sort(w.begin(), w.end(), std::greater<uint64_t>());
-            for (int i = 0; i < L.n_pairs; ++i) po[i] = 0xffffff - (int)(w[i] & 0xffffff);
-        }
-        if (!b->pairs2.empty()) { std::vector<nr::pr::Pair2> t(L.n_pairs); for (int i = 0; i < L.n_pairs; ++i) t[i] = b->pairs2[po[i]]; b->pairs2.swap(t); }
-        else { std::vector<nr::pr::Pair3> t(L.n_pairs); for (int i = 0; i < L.n_pairs; ++i) t[i] = b->pairs3[po[i]]; b->pairs3.swap(t); }
-        for (long long c : pair_cost) b->paired_cells += 2 * c;             // both halves of every word
-        b->stats.executed_cells += b->paired_cells;
-        L.pair_blocks = std::max(1, std::min(g_ctx.sm_count, L.n_pairs));
-    }
-    trace.mark("pair order");
-    b->n_pairs2_single = (int)b->pairs2.size();
-    // ---- pairs of LONG reads (round 2): two reads of a region that are longer than one paired stripe share the u16x2
-    // words stripe by stripe; their stripes are cooperative entries like the 32-bit ones.  A read pairs with the next
-    // shorter one of its region if that one is at least half as long (the pair sweeps the longer read's rows).
-    struct LongPair { int a, b, n_left; long long cost; };
-    std::vector<LongPair> long_pairs;
-    long long long_pair_rows = 0;
-    b->n_pairs3_single = (int)b->pairs3.size();
-    if (b->pair && fixed && ladder && b->flag && !getenv("NR_NO_LONG_PAIRS")) {
-        // round 3: the same, over the reads that have a ladder; the pair sweeps the union of the two ladders
-        for (int i0 = 0; i0 < n;) {
-            int i1 = i0;
-            while (i1 < n && b->ltasks[i1].region == b->ltasks[i0].region) ++i1;
-            const nr::LadderRegion& g = b->lregs[b->ltasks[i0].region];
-            std::vector<int> ids;
-            if (g.n_left > 0 && g.n_right > 0)
-                for (int i = i0; i < i1; ++i)
-                    if (!paired[i] && b->ltasks[i].q_len > 32 * nr::pr::kMaxRPair3) ids.push_back(i);
-            std::sort(ids.begin(), ids.end(), [&](int x, int y) { return b->ltasks[x].q_len != b->ltasks[y].q_len ? b->ltasks[x].q_len > b->ltasks[y].q_len : x < y; });
-            for (size_t i = 0; i + 1 < ids.size();) {
-                const int x = ids[i], y = ids[i + 1];
-                if (2 * b->ltasks[y].q_len >= b->ltasks[x].q_len) {
-                    long_pairs.push_back({x, y, g.n_left, 0});
-                    paired[x] = paired[y] = 3;
-                    long_pair_rows += b->ltasks[x].q_len;
-                    i += 2;
-                } else {
-                    ++i;
-                }
-            }
-            i0 = i1;
-        }
-    }
-    if (b->pair && fixed && !ladder && b->kind == KIND_ROUND2 && !getenv("NR_NO_LONG_PAIRS")) {
-        for (const RegionInfo& g : b->regions) {
-            std::vector<int> ids;
-            for (int r = g.first_read; r < g.first_read + g.n_reads; ++r)
-                if (!paired[r] && b->tasks[r].q_len > 32 * nr::pr::kMaxRPair2 && b->tasks[r].t_len >= 1) ids.push_back(r);
-            std::sort(ids.begin(), ids.end(), [&](int x, int y) { return b->tasks[x].q_len != b->tasks[y].q_len ? b->tasks[x].q_len > b->tasks[y].q_len : x < y; });
-            for (size_t i = 0; i + 1 < ids.size();) {
-                const int x = ids[i], y = ids[i + 1];
-                if (2 * b->tasks[y].q_len >= b->tasks[x].q_len) {
-                    long_pairs.push_back({x, y, g.n_left, 0});
-                    paired[x] = paired[y] = 3;
-                    long_pair_rows += b->tasks[x].q_len;
-                    i += 2;
-                } else {
-                    ++i;
-                }
-            }
-        }
-    }
-    // ---- the rest: one persistent launch of the 32-bit kernels.  Long reads are cut into stripes that run on
-    // different warps at the same time (nr_kernels.cuh, CoopInfo); their entries come first, by decreasing cost, every
-    // entry behind what it waits for; then the single-stripe tasks by decreasing cost ----
-    std::vector<int> singles, multis;
-    long long multi_rows = 0;
-    for (int i = 0; i < n; ++i) {
-        if (paired[i]) continue;
-        (task_ns[i] > 1 ? multis : singles).push_back(i);
-        if (task_ns[i] > 1) multi_rows += ladder ? b->ltasks[i].q_len : b->tasks[i].q_len;
-    }
-    int coop_height = 12;
-    if (!multis.empty() || !long_pairs.empty()) {
-        // stripe height of the long tasks: the shortest that does not cut them into more stripes than there are warps
-        // to run them side by side (a stripe is one warp's work; the ladder's two sweeps overlap)
-        const long long warps = (long long)kWarpsPerBlock * g_ctx.sm_count;
-        int cap = max_r;
-        const char* force = getenv("NR_COOP_ROWS");       // tuning / debugging: fixed stripe height of the long tasks
-        if (force && atoi(force) >= nr::kMinR && atoi(force) <= max_r) cap = std::min(nr::coop_height_at_least(atoi(force)), max_r);
-        else for (int r : {4, 6, 8}) {
-            if (r >= max_r) break;
-            const long long stripes = ((multi_rows + long_pair_rows) / (32 * r) + (long long)multis.size() + (long long)long_pairs.size()) * (ladder ? 2 : 1);
-            if (stripes <= warps) { cap = r; break; }
-        }
-        // ONE stripe height for all long tasks of the batch.  Every height is its own unrolled code; long reads running
-        // at six different heights at once miss the instruction cache on most fetches (config 5: 4.7 stall cycles per
-        // issued instruction, round 3 in 183 ms with three heights in flight against 57 ms with one).  The last stripe of
-        // a task is padded up to the common height.
-        const int height = std::min(cap, 12);
-        coop_height = height;
-        for (int i : multis) {
-            const int q_len = ladder ? b->ltasks[i].q_len : b->tasks[i].q_len;
-            int R = height, ns = (q_len + 32 * height - 1) / (32 * height);
-            if (ns > nr::kCodeFwd - 2) {                            // too long for that many stripes: its own, taller ones
-                R = nr::coop_height_at_least(nr::coop_rows(q_len, nr::kCodeFwd - 2));
-                ns = (q_len + 32 * R - 1) / (32 * R);
-            }
-            if (R > max_r)
-                return fail(NR_ERR_TOO_LARGE, "task %d: a query of %d bases needs more than %d stripes", i, q_len, nr::kCodeFwd - 2);
-            cost[i] = cost[i] / ((long long)task_ns[i] * task_R[i]) * ((long long)ns * R);
-            task_ns[i] = ns;
-            task_R[i] = R;
-        }
-    }
-    // long pairs at the common height; one that would need more than 62 stripes goes back to the 32-bit kernels
-    {
-        std::vector<LongPair> keep;
-        auto qlen_of = [&](int t) { return ladder ? b->ltasks[t].q_len : b->tasks[t].q_len; };
-        for (LongPair& lp : long_pairs) {
-            const int q = qlen_of(lp.a), ns = (q + 32 * coop_height - 1) / (32 * coop_height);
-            if (ns > nr::kCodeFwd - 2 || b->pairs2.size() + b->pairs3.size() + keep.size() >= (1u << 22)) {
-                for (int t : {lp.a, lp.b}) {
-                    paired[t] = 0;
-                    multis.push_back(t);
-                    int R = nr::coop_height_at_least(nr::coop_rows(qlen_of(t), nr::kCodeFwd - 2));
-                    R = std::max(R, coop_height);
-                    const int ns1 = (qlen_of(t) + 32 * R - 1) / (32 * R);
-                    cost[t] = cost[t] / ((long long)task_ns[t] * task_R[t]) * ((long long)ns1 * R);
-                    task_ns[t] = ns1; task_R[t] = R;
-                }
-                continue;
-            }
-            long long cols;
-            if (ladder) {
-                const nr::LadderRegion& g = b->lregs[b->ltasks[lp.a].region];
-                cols = (long long)g.n_right + g.n_left + (long long)g.m * std::max(b->ltasks[lp.a].kmax, b->ltasks[lp.b].kmax);
-            } else {
-                cols = b->tasks[lp.a].t_len;
-            }
-            lp.cost = (long long)ns * 32 * coop_height * cols;
-            keep.push_back(lp);
-        }
-        long_pairs.swap(keep);
-        std::sort(long_pairs.begin(), long_pairs.end(), [](const LongPair& x, const LongPair& y) { return x.cost != y.cost ? x.cost > y.cost : x.a < y.a; });
-    }
-    int rmax = 0;
-    for (int i = 0; i < n; ++i) {
-        if (paired[i]) continue;
-        rmax = std::max(rmax, task_R[i]);
-        b->rest_cells += cost[i];
-        b->rest_useful += cost[i] / ((long long)task_ns[i] * 32 * task_R[i]) * (ladder ? b->ltasks[i].q_len : b->tasks[i].q_len);
-    }
-    b->stats.executed_cells += b->rest_cells;
-    auto by_cost = [&](int x, int y) { return cost[x] != cost[y] ? cost[x] > cost[y] : x < y; };
-    std::sort(singles.begin(), singles.end(), by_cost);
-    std::sort(multis.begin(), multis.end(), by_cost);
-    if (n > (1 << (31 - nr::kCodeBits))) return fail(NR_ERR_TOO_LARGE, "more than 2^24 tasks in one batch");
-    b->order.clear();
-    b->coop.clear();
-    if (!ladder) b->coop_idx.assign(n, -1);
-    long long data_off = 0, flag_off = 0;
-    for (int i : multis) {
-        nr::CoopInfo ci = {};
-        ci.n_stripes = task_ns[i];
-        ci.rows = task_R[i];
-        ci.data_off = data_off;
-        ci.flag_off = (int)flag_off;
-        ci.bnd_stride = (task_sweep[i] + 63) / 32 * 32;
-        if (ladder) {
-            ci.b_stride = task_ns[i] * 32 * task_R[i];
-            ci.tok_stride = (task_rungs[i] + 1) / 2 * 2;
-        }
-        data_off += (ladder ? 4LL : 2LL) * ci.bnd_stride + ci.b_stride + 2LL * ci.tok_stride;
-        flag_off += nr::kCoopFlagInts(task_ns[i]);
-        if (flag_off > 0x7fffffffLL) return fail(NR_ERR_TOO_LARGE, "too many long tasks in one batch");
-        if (ladder) b->ltasks[i].pad = (int32_t)b->coop.size();
-        else b->coop_idx[i] = (int32_t)b->coop.size();
-        b->coop.push_back(ci);
-    }
-    std::vector<int> long_pair_ns;
-    for (const LongPair& lp : long_pairs) {
-        if (ladder) {
-            const nr::LadderTask& ta = b->ltasks[lp.a];
-            const nr::LadderTask& tb = b->ltasks[lp.b];
-            const nr::LadderRegion& g = b->lregs[ta.region];
-            const int kmin = std::min(ta.kmin, tb.kmin), kmax = std::max(ta.kmax, tb.kmax), rungs = kmax - kmin + 1;
-            nr::CoopInfo ci = {};
-            ci.n_stripes = (ta.q_len + 32 * coop_height - 1) / (32 * coop_height);
-            ci.rows = coop_height;
-            ci.data_off = data_off;
-            ci.flag_off = (int)flag_off;
-            ci.bnd_stride = (std::max(g.n_left + g.m * kmax, g.n_right) + 63) / 32 * 32;
-            ci.b_stride = ci.n_stripes * 32 * coop_height;          // words per plane of the backward stripes' junction state
-            ci.tok_stride = (rungs + 1) / 2 * 2;
-            data_off += 4LL * ci.bnd_stride + (3LL * ci.b_stride + 3) / 4 + 2LL * ci.tok_stride;
-            flag_off += nr::kCoopFlagInts(ci.n_stripes);
-            if (flag_off > 0x7fffffffLL) return fail(NR_ERR_TOO_LARGE, "too many long tasks in one batch");
-            nr::pr::Pair3 p = {lp.a, lp.b, (int32_t)rung_off, -1, coop_height, {(int32_t)b->coop.size(), 0, 0}};
-            rung_off += rungs;
-            b->coop.push_back(ci);
-            b->pairs3.push_back(p);
-            long_pair_ns.push_back(ci.n_stripes);
-            L.pair_R = std::max(L.pair_R, coop_height);
-            b->paired_cells += 2 * lp.cost;
-            b->stats.executed_cells += 2 * lp.cost;
-            b->paired_useful += (long long)(ta.q_len + tb.q_len) * (lp.cost / ((long long)ci.n_stripes * 32 * coop_height));
-            continue;
-        }
-        const nr::Task& ta = b->tasks[lp.a];
-        nr::CoopInfo ci = {};
-        ci.n_stripes = (ta.q_len + 32 * coop_height - 1) / (32 * coop_height);
-        ci.rows = coop_height;
-        ci.data_off = data_off;
-        ci.flag_off = (int)flag_off;
-        ci.bnd_stride = (ta.t_len + 63) / 32 * 32;
-        data_off += 2LL * ci.bnd_stride;
-        flag_off += nr::kCoopFlagInts(ci.n_stripes);
-        if (flag_off > 0x7fffffffLL) return fail(NR_ERR_TOO_LARGE, "too many long tasks in one batch");
-        nr::pr::Pair2 p = {lp.a, lp.b, lp.n_left, (int32_t)b->coop.size()};      // state_off = the pair's CoopInfo
-        b->coop.push_back(ci);
-        b->pairs2.push_back(p);
-        long_pair_ns.push_back(ci.n_stripes);
-        L.pair_R = std::max(L.pair_R, coop_height);
-        b->paired_cells += 2 * lp.cost;
-        b->stats.executed_cells += 2 * lp.cost;
-        b->paired_useful += (long long)(ta.q_len + b->tasks[lp.b].q_len) * ta.t_len;
-    }
-    b->n_long_pairs = (int)long_pairs.size();
-    if (rung_off > 0x7fffffffLL) return fail(NR_ERR_TOO_LARGE, "more than 2^31 rungs in one batch");
-    if (!b->pairs3.empty()) b->prung_bytes = sizeof(uint2) * (size_t)std::max<long long>(rung_off, 1);
-    // Stripe-major: stripe 0 of every long task, then stripe 1 of every long task, ...  A stripe waits for the one above
-    // it; listed task by task, all stripes of a task would be picked up at the same moment and stripe s would spin for
-    // s x (lag of ~95 columns) before its first column -- with 20 stripes over the 1000 columns of the right anchor
-    // that is more waiting than work (measured on config 5: a fifth of all executed instructions were retry loops).
-    // Level by level, a stripe is picked up when the one above it is well under way or done, and the parallelism comes
-    // from the tasks; with few long tasks all levels are in flight at once and the stripes pipeline as before.
-    int max_ns = 0;
-    for (int i : multis) max_ns = std::max(max_ns, task_ns[i]);
-    for (int ns : long_pair_ns) max_ns = std::max(max_ns, ns);
-    for (int st = 0; st < max_ns; ++st) {                   // first sweep of every long task (ladder: backward)
-        for (size_t k = 0; k < long_pair_ns.size(); ++k)    // (pairs of long reads: entries point into pairs[])
-            if (st < long_pair_ns[k])
-                b->order.push_back(nr::pr::kPairEntry | (((ladder ? b->n_pairs3_single : b->n_pairs2_single) + (int)k) << nr::kCodeBits) | (1 + st));
-        for (int i : multis) {
-            if (st >= task_ns[i] || (ladder && b->lregs[b->ltasks[i].region].n_right == 0)) continue;
-            b->order.push_back((i << nr::kCodeBits) | (1 + st));
-        }
-    }
-    if (ladder)
-        for (int st = 0; st < max_ns; ++st) {
-            for (size_t k = 0; k < long_pair_ns.size(); ++k)
-                if (st < long_pair_ns[k])
-                    b->order.push_back(nr::pr::kPairEntry | ((b->n_pairs3_single + (int)k) << nr::kCodeBits) | (nr::kCodeFwd + st));
-            for (int i : multis)
-                if (st < task_ns[i]) b->order.push_back((i << nr::kCodeBits) | (nr::kCodeFwd + st));
-        }
-    for (int i : singles) b->order.push_back(i << nr::kCodeBits);
-    const int n_rest = (int)b->order.size();
-    L.ladder = ladder;
-    L.R = rmax;
-    L.count = n_rest;
-    // one persistent block per SM (every block resident: entries may wait for each other); a small batch still spreads
-    L.blocks = std::max(1, std::min(g_ctx.sm_count, n_rest));
-    L.fixed = fixed;
-    const size_t scratch_total = (size_t)data_off;
-    b->flags_bytes = sizeof(int) * (size_t)flag_off;
-    trace.mark("32-bit entries");
-    // ---- one device blob: [tasks | regions | order | pairs | pool (+4 slack words) | counters], staged in pinned memory ----
-    const size_t task_bytes = ladder ? sizeof(nr::LadderTask) * n : sizeof(nr::Task) * n;
-    const size_t reg_bytes = sizeof(nr::LadderRegion) * b->lregs.size();
-    const size_t order_bytes = sizeof(int32_t) * n_rest;
-    const size_t pair_bytes = b->pairs2.empty() ? sizeof(nr::pr::Pair3) * b->pairs3.size() : sizeof(nr::pr::Pair2) * b->pairs2.size();
-    const size_t pool_bytes = sizeof(uint32_t) * (b->pool.words.size() + 4);
-    const size_t coop_bytes = sizeof(nr::CoopInfo) * b->coop.size();
-    const size_t cidx_bytes = b->coop.empty() ? 0 : sizeof(int32_t) * b->coop_idx.size();
-    const size_t off_reg = align_up(task_bytes, 256);
-    const size_t off_order = off_reg + align_up(reg_bytes, 256);
-    const size_t off_pair = off_order + align_up(order_bytes, 256);
-    const size_t off_coop = off_pair + align_up(pair_bytes, 256);
-    const size_t off_cidx = off_coop + align_up(coop_bytes, 256);
-    const size_t off_pool = off_cidx + align_up(cidx_bytes, 256);
-    const size_t off_cnt = off_pool + align_up(pool_bytes, 256);
-    b->blob_bytes = off_cnt + 256;
-    b->out_bytes = sizeof(int4) * std::max<size_t>(b->n_out, 1);
-    b->scratch_bytes = sizeof(int4) * scratch_total;
     int rc;
     if ((rc = cached_alloc(&b->d_blob, b->blob_bytes, BUF_DEV))) return rc;
     if ((rc = cached_alloc(&b->h_blob, b->blob_bytes, BUF_PIN))) return rc;
     if ((rc = cached_alloc((void**)&b->d_out, b->out_bytes, BUF_DEV))) return rc;
     if ((rc = cached_alloc((void**)&b->h_out, b->out_bytes, BUF_PIN))) return rc;
-    if (scratch_total && (rc = cached_alloc((void**)&b->d_scratch, b->scratch_bytes, BUF_SCRATCH))) return rc;
+    if (b->scratch_bytes && (rc = cached_alloc((void**)&b->d_scratch, b->scratch_bytes, BUF_SCRATCH))) return rc;
     if (b->flags_bytes && (rc = cached_alloc((void**)&b->d_flags, b->flags_bytes, BUF_DEV))) return rc;
     if (b->state_bytes && (rc = cached_alloc((void**)&b->d_state, b->state_bytes, BUF_DEV))) return rc;
     if (b->round2_exit &&
         (rc = cached_alloc((void**)&b->d_kept, sizeof(uint32_t) * 128 * kWarpsPerBlock * (size_t)g_ctx.sm_count, BUF_DEV))) return rc;
     if (b->flag) {
-        b->sel_bytes = sizeof(int4) * std::max<size_t>((size_t)b->n_reads, 1);
         if ((rc = cached_alloc((void**)&b->d_sel, b->sel_bytes, BUF_DEV))) return rc;
         if ((rc = cached_alloc((void**)&b->h_sel, b->sel_bytes, BUF_PIN))) return rc;
     }
     if (!b->pairs3.empty()) {
-        b->redo_bytes = sizeof(int32_t) * (size_t)n * 2;       // [n] entries of the device-side redo launch | [n] long reads for the host
         if ((rc = cached_alloc((void**)&b->d_prung, b->prung_bytes, BUF_DEV))) return rc;
         if ((rc = cached_alloc((void**)&b->d_redo, b->redo_bytes, BUF_DEV))) return rc;
         if ((rc = cached_alloc((void**)&b->h_redo_count, 64, BUF_PIN))) return rc;
@@ -926,36 +320,34 @@ int plan_batch(nr_batch* b) {
     trace.mark("buffers (cached alloc)");
     char* h = static_cast<char*>(b->h_blob);
     char* d = static_cast<char*>(b->d_blob);
-    if (task_bytes) memcpy(h, ladder ? (const void*)b->ltasks.data() : (const void*)b->tasks.data(), task_bytes);
-    if (reg_bytes) memcpy(h + off_reg, b->lregs.data(), reg_bytes);
-    if (order_bytes) memcpy(h + off_order, b->order.data(), order_bytes);
-    if (coop_bytes) memcpy(h + off_coop, b->coop.data(), coop_bytes);
-    if (cidx_bytes) memcpy(h + off_cidx, b->coop_idx.data(), cidx_bytes);
-    if (pair_bytes) memcpy(h + off_pair, b->pairs2.empty() ? (const void*)b->pairs3.data() : (const void*)b->pairs2.data(), pair_bytes);
-    if (!b->pool.words.empty()) memcpy(h + off_pool, b->pool.words.data(), pool_bytes - 16);
-    memset(h + off_pool + pool_bytes - 16, 0, 16);
-    memset(h + off_cnt, 0, 256);
-    b->d_tasks = reinterpret_cast<nr::Task*>(d);
-    b->d_ltasks = reinterpret_cast<nr::LadderTask*>(d);
-    b->d_lregs = reinterpret_cast<nr::LadderRegion*>(d + off_reg);
-    b->d_order = reinterpret_cast<int32_t*>(d + off_order);
-    b->d_pairs = d + off_pair;
-    b->d_coop = reinterpret_cast<nr::CoopInfo*>(d + off_coop);
-    b->d_coop_idx = reinterpret_cast<int32_t*>(d + off_cidx);
-    b->d_pool = reinterpret_cast<uint32_t*>(d + off_pool);
-    b->d_counters = reinterpret_cast<int*>(d + off_cnt);
+    for (const Section& s : b->blob) {
+        if (s.bytes) memcpy(h + s.off, s.src, s.bytes);
+        memset(h + s.off + s.bytes, 0, s.zeros);
+    }
+    memset(h + b->blob_bytes - 256, 0, 256);
+    b->d_tasks = reinterpret_cast<nr::Task*>(d + b->blob[SEC_TASKS].off);
+    b->d_ltasks = reinterpret_cast<nr::LadderTask*>(d + b->blob[SEC_TASKS].off);
+    b->d_lregs = reinterpret_cast<nr::LadderRegion*>(d + b->blob[SEC_LREGS].off);
+    b->d_order = reinterpret_cast<int32_t*>(d + b->blob[SEC_ORDER].off);
+    b->d_pairs = d + b->blob[SEC_PAIRS].off;
+    b->d_coop = reinterpret_cast<nr::CoopInfo*>(d + b->blob[SEC_COOP].off);
+    b->d_coop_idx = reinterpret_cast<int32_t*>(d + b->blob[SEC_COOP_IDX].off);
+    b->d_pool = reinterpret_cast<uint32_t*>(d + b->blob[SEC_POOL].off);
+    b->d_counters = reinterpret_cast<int*>(d + b->blob_bytes - 256);
     trace.mark("blob staging (memcpy)");
     cudaStream_t st = g_ctx.stream;
     CUDA_TRY(cudaMemcpyAsync(d, h, b->blob_bytes, cudaMemcpyHostToDevice, st));
     CUDA_TRY(cudaMemsetAsync(b->d_out, 0, b->out_bytes, st));
     if (b->d_sel) CUDA_TRY(cudaMemsetAsync(b->d_sel, 0, b->sel_bytes, st));
     CUDA_TRY(cudaEventRecord(b->ev_uploaded, st));      // nr_batch_run on another stream waits for it; no host sync here
-    b->stats.h2d_bytes = (int64_t)(task_bytes + reg_bytes + order_bytes + pair_bytes + coop_bytes + cidx_bytes + pool_bytes);
-    b->stats.d2h_bytes = (int64_t)sizeof(int4) * (b->flag ? (int64_t)b->n_reads : (int64_t)b->n_out);
-    b->stats.n_skipped = b->n_skipped;
     trace.mark("upload + memsets (async)");
     b->committed = true;
     return NR_OK;
+}
+
+int commit_batch(nr_batch* b) {
+    const int rc = plan_batch(b, g_ctx.sm_count);
+    return rc ? rc : upload_batch(b);
 }
 
 constexpr int kSpinSlot = 16;        // d_counters[kSpinSlot]: the batch's give-up flag (nr_kernels.cuh, wait_cols)
@@ -1429,7 +821,7 @@ int redo_long_reads(nr_batch* b) {
     }
     t->n_reads = cnt;
     t->n_out = (size_t)t->rung_off.back();
-    int rc = plan_batch(t);
+    int rc = commit_batch(t);
     if (!rc) rc = run_batch(t, st);
     if (!rc) rc = fetch_raw(t);
     if (!rc)
@@ -1603,7 +995,7 @@ int nr_batch_add_round3(nr_batch_t* b, const char* left, int32_t n_left, const c
 
 int nr_batch_commit(nr_batch_t* b) {
     if (!b || b->committed) return fail(NR_ERR_ARG, "nr_batch_commit: NULL or already committed batch");
-    return plan_batch(b);
+    return commit_batch(b);
 }
 
 nr_batch_t* nr_batch_create_tasks(const nr_scoring_t* sc, int32_t n_tasks, const char* const* queries,
@@ -1634,7 +1026,7 @@ nr_batch_t* nr_batch_create_tasks(const nr_scoring_t* sc, int32_t n_tasks, const
         t.q_word = words[0];
         t.t_word = words[1];
     }
-    if (plan_batch(b)) { nr_batch_destroy(b); return nullptr; }
+    if (commit_batch(b)) { nr_batch_destroy(b); return nullptr; }
     return b;
 }
 
@@ -1645,7 +1037,7 @@ nr_batch_t* nr_batch_create_round2(const nr_scoring_t* sc, const char* left, int
     nr_batch* b = new_batch(sc, KIND_ROUND2);
     if (!b) return nullptr;
     ReadSrc src = {cores, core_len, nullptr, nullptr, 0};
-    if (add_round2(b, left, n_left, motif, motif_len, T, n_reads, src) || plan_batch(b)) { nr_batch_destroy(b); return nullptr; }
+    if (add_round2(b, left, n_left, motif, motif_len, T, n_reads, src) || commit_batch(b)) { nr_batch_destroy(b); return nullptr; }
     return b;
 }
 
@@ -1657,7 +1049,7 @@ nr_batch_t* nr_batch_create_round3(const nr_scoring_t* sc, const char* left, int
     nr_batch* b = new_batch(sc, KIND_ROUND3);
     if (!b) return nullptr;
     ReadSrc src = {cores, core_len, nullptr, nullptr, 0};
-    if (add_round3(b, left, n_left, right, n_right, motif, motif_len, n_reads, src, kmin, kmax) || plan_batch(b)) {
+    if (add_round3(b, left, n_left, right, n_right, motif, motif_len, n_reads, src, kmin, kmax) || commit_batch(b)) {
         nr_batch_destroy(b);
         return nullptr;
     }
@@ -2124,7 +1516,6 @@ extern "C" int nr_estimate_regions(const nr_scoring_t* sc, int32_t fast_mode, in
 }
 
 // ---- what the other host translation units (nr_joint.cu, nr_anchor.cu) share with this one ----------------------------
-#include "nr_internal.h"
 namespace nri {
 int ensure_init() { return ::ensure_init(-1); }
 cudaStream_t stream() { return g_ctx.stream; }

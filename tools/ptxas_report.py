@@ -1,25 +1,30 @@
 #!/usr/bin/env python
-"""Compile nr_api.cu with -Xptxas -v and print one line per kernel: registers, spills, smem."""
-import re, subprocess, sys, os
+"""Registers, stack frame, local and shared memory per kernel of the built library, from `cuobjdump -res-usage`.
+
+usage: ptxas_report.py [path/to/libnanorepeat_b200.so]   (default: the in-tree library that `make` builds)
+
+One line per kernel, sorted by name, so that two builds compare with `diff`.  Spills live in the stack frame:
+cuobjdump reports no separate spill count (`nvcc -Xptxas -v` does, per translation unit)."""
+import os
+import re
+import subprocess
+import sys
+
 here = os.path.dirname(os.path.abspath(__file__))
-src = os.path.join(here, "..", "nanorepeat_b200", "csrc", "nr_api.cu")
-out = subprocess.run(["/usr/local/cuda/bin/nvcc", "-gencode", "arch=compute_100a,code=sm_100a", "-O3", "-lineinfo",
-                      "-std=c++17", "-Xcompiler", "-fPIC", "-Xptxas", "-v", "-shared", "-o", "/tmp/_ptxas_report.so", src]
-                     + sys.argv[1:], capture_output=True, text=True).stderr
-cur = None
-rows = {}
+lib = sys.argv[1] if len(sys.argv) > 1 else os.path.join(here, "..", "nanorepeat_b200", "libnanorepeat_b200.so")
+out = subprocess.run(["/usr/local/cuda/bin/cuobjdump", "-res-usage", lib], capture_output=True, text=True, check=True).stdout
+rows, name = {}, None
 for ln in out.splitlines():
-    m = re.search(r"Compiling entry function '(\S+)'", ln)
+    m = re.match(r"\s*Function (\S+):$", ln)
     if m:
-        d = subprocess.run(["c++filt", m.group(1)], capture_output=True, text=True).stdout
-        mm = re.search(r"nr::(\w+)<(true|false)>", d)
-        cur = (mm.group(1), mm.group(2) == "true", 0) if mm else (m.group(1), False, 0)
-        rows[cur] = {}
-    m = re.search(r"(\d+) bytes stack frame, (\d+) bytes spill stores, (\d+) bytes spill loads", ln)
-    if m and cur:
-        rows[cur]["stack"], rows[cur]["spill"] = int(m.group(1)), int(m.group(2))
-    m = re.search(r"Used (\d+) registers", ln)
-    if m and cur:
-        rows[cur]["regs"] = int(m.group(1))
+        d = subprocess.run(["c++filt", m.group(1)], capture_output=True, text=True).stdout.strip()
+        d = d.replace("(anonymous namespace)::", "")
+        name = re.sub(r"^void ", "", d.split("(")[0])       # drop the parameter list: templates name the variant
+        continue
+    if name:
+        f = dict(re.findall(r"(\w+(?:\[\d+\])?):(\d+)", ln))
+        rows[name] = f"regs={f.get('REG')} stack={f.get('STACK')} local={f.get('LOCAL')} shared={f.get('SHARED')}"
+        name = None
+width = max(map(len, rows), default=0)
 for k in sorted(rows):
-    print(f"{k[0]:14s} multi={int(k[1])} R={k[2]:2d} regs={rows[k].get('regs')} stack={rows[k].get('stack')} spill={rows[k].get('spill')}")
+    print(f"{k:{width}s}  {rows[k]}")
