@@ -268,7 +268,9 @@ int nr_estimate_regions(const nr_scoring_t* sc, int32_t fast_mode, int32_t n_reg
  * [left.qend - 100, right.qstart + 100) clamped to the read, the middle [left.qend, right.qstart) (:221-234), both in
  * the orientation of the left anchor's strand.  Two kernel launches per call, whatever the number of regions.
  * A read that is empty, longer than nr_limits' template limit or holds a character other than ACGTacgt is not scored
- * (no hit; nr_stats_t.n_skipped counts the last two); an anchor may hold any character (N scores -ambiguous).
+ * (no hit; nr_stats_t.n_skipped counts the last two); an anchor may hold any character (N scores -ambiguous).  An anchor
+ * whose score can exceed nr_limits' score limit on a read (match * min(|anchor|, |read|) > 32767) is not scored on that
+ * read: it has no hit there, and n_skipped counts each such (read, anchor) once.
  * Needs map-ont scoring with min_dp_score >= 10 * match (every preset): a hit then spans >= 10 read bases, so the
  * reference's align_len < 10 test (:173) never decides.
  */
@@ -291,7 +293,8 @@ typedef struct nr_anchor_read_t {           /* one per read, concatenated in reg
                                                qstart is recovered for good anchors only (-1 otherwise) */
 } nr_anchor_read_t;
 int nr_anchor_regions(const nr_scoring_t* sc, int32_t n_regions, const nr_anchor_region_t* regions, nr_anchor_read_t* out,
-                      nr_stats_t* stats /* nullable: algorithmic cells = sum of 2 * (|left| + |right|) * |read| */);
+                      nr_stats_t* stats /* nullable: algorithmic cells = sum of 2 * (|left| + |right|) * |read| over the
+                                           scored reads */);
 
 /*
  * Joint path (nanoRepeat-joint: two neighbouring repeats quantified together).  The reference aligns every read against

@@ -11,7 +11,8 @@
 //      l * min(e, e2) + min(q, q2)), and tend is the smallest end reaching S on the whole strand, so every alignment of
 //      the window that reaches S ends at tend: the window's record is (S, tstart - a, tend - a) with the contract's
 //      tie-break.  The library checks score and end and fails the call rather than return another start.
-//      Anchors too long for a 16-bit half are scored here too, against whole strands.
+//      Anchors too long for a 16-bit half are scored here too, against whole strands; where even a 32-bit task cannot
+//      hold the score (match * min(|anchor|, |read|) > 32767) the anchor gets no hit on that read and n_skipped counts it.
 // Then the reference's rules, on the host.
 #include "nr_batch.h"
 #include "nr_internal.h"
@@ -141,12 +142,12 @@ int anchor_regions(const nr_scoring_t* sc, int n_regions, const nr_anchor_region
     for (int g = 0; g < n_regions; ++g) {
         const nr_anchor_region_t& G = regs[g];
         const int qa = G.n_left <= kMaxPairAnchor ? G.n_left : 0, qb = G.n_right <= kMaxPairAnchor ? G.n_right : 0;
-        if (qa == 0 && qb == 0) continue;
-        int R, S;
-        pair_shape(std::max(qa, qb), R, S);
+        int R = 0, S = 0;
+        if (qa > 0 || qb > 0) pair_shape(std::max(qa, qb), R, S);
         for (long long i = first[g]; i < first[g + 1]; ++i) {
             if (fwd_word[i] < 0) continue;
-            for (int sd = 0; sd < 2; ++sd) {
+            st.algorithmic_cells += 2LL * ((long long)G.n_left + G.n_right) * rlen[i];    // long anchors included
+            for (int sd = 0; sd < 2 && S > 0; ++sd) {
                 nr::pr::AnchorPair p = {};
                 p.t_word = (uint32_t)(sd ? rev_word[i] : fwd_word[i]); p.t_len = rlen[i];
                 p.qa_word = (uint32_t)left_word[g]; p.q_a = qa;
@@ -157,7 +158,6 @@ int anchor_regions(const nr_scoring_t* sc, int n_regions, const nr_anchor_region
                 if (S > 1) max_multi_t = std::max(max_multi_t, rlen[i]);
                 st.executed_cells += 2LL * 32 * R * S * rlen[i];
             }
-            st.algorithmic_cells += 2LL * ((long long)G.n_left + G.n_right) * rlen[i];
         }
     }
     const int n_pairs = (int)pairs.size();
@@ -243,6 +243,10 @@ int anchor_regions(const nr_scoring_t* sc, int n_regions, const nr_anchor_region
             for (long long i = first[g]; i < first[g + 1]; ++i) {
                 if (fwd_word[i] < 0 || n == 0) continue;
                 if (n > kMaxPairAnchor) {
+                    if ((long long)sc->match * std::min(n, rlen[i]) > nrh::kMaxScore) {     // no DP word holds its score:
+                        ++st.n_skipped;                                                     // no hit, counted once
+                        continue;
+                    }
                     for (int sd = 0; sd < 2; ++sd) {
                         tq.push_back(q); tql.push_back(n);
                         tt.push_back(sd ? rev[i].data() : rptr[i]); ttl.push_back(rlen[i]);
@@ -274,12 +278,11 @@ int anchor_regions(const nr_scoring_t* sc, int n_regions, const nr_anchor_region
         nr_batch_destroy(b);
         if (rc) return rc;
         st.executed_cells += bs.executed_cells; st.n_tasks += bs.n_tasks; st.kernel_launches += bs.kernel_launches;
-        st.h2d_bytes += bs.h2d_bytes; st.d2h_bytes += bs.d2h_bytes;
+        st.n_skipped += bs.n_skipped; st.h2d_bytes += bs.h2d_bytes; st.d2h_bytes += bs.d2h_bytes;
         for (int t = 0; t < nt; ++t) {
             Cand& c = cand[tslot[t]];
-            if (twin[t] < 0) {             // a whole strand (long anchor): the record as it is
+            if (twin[t] < 0) {             // a whole strand (long anchor): the record as it is (tstart kept for good anchors)
                 c.score = res[t].score; c.tstart = res[t].tstart; c.tend = res[t].tend;
-                st.algorithmic_cells += (long long)tql[t] * ttl[t];
                 continue;
             }
             if (res[t].score != c.score || res[t].tend != c.tend - twin[t]) {
@@ -307,7 +310,8 @@ int anchor_regions(const nr_scoring_t* sc, int n_regions, const nr_anchor_region
             best[a]->tstart = -1;
             if (nh[a]) {
                 const Cand& c = cand[4 * i + 2 * a + idx[a][0]];
-                best[a]->score = c.score; best[a]->tstart = c.tstart; best[a]->tend = c.tend;
+                best[a]->score = c.score; best[a]->tend = c.tend;
+                if (ok[a]) best[a]->tstart = c.tstart;                    // whole-strand records carry one either way
                 *strand[a] = idx[a][0] ? '-' : '+';
             }
         }
