@@ -16,7 +16,7 @@ from .repeat_region import Read, RepeatRegion                                  #
 from .estimation import (round1_and_round2_estimation, round3_estimation,     # noqa: F401
                          round3_estimation_for1read, estimate_regions, install)
 from . import engine, sharding, pymm2_shim, joint, anchoring, phasing          # noqa: F401
-from .sharding import estimate_regions_sharded                                 # noqa: F401
+from .sharding import estimate_regions_sharded, quantify_regions_sharded       # noqa: F401
 from .pipeline import quantify_regions                                         # noqa: F401
 
 __version__ = "0.1.0"

@@ -93,26 +93,43 @@ def find_anchor_locations_in_regions(data_type, repeat_regions, region_reads, re
     a = 0
     for rr, (names, _seqs) in zip(repeat_regions, named):
         end = first + len(names)
+        rows = []
         while a < len(accepted) and accepted[a] < end:
-            i = accepted[a]
+            rows.append(accepted[a])
             a += 1
-            name = names[i - first]
-            read = read_class()
-            read.read_name = name
-            read.full_read_len = col["read_len"][i]
-            read.left_anchor_is_good = read.right_anchor_is_good = read.both_anchors_are_good = True
-            read.left_anchor_paf = AnchorHit(chr(col["left_strand"][i]), col["leftscore"][i], col["lefttstart"][i], col["lefttend"][i])
-            read.right_anchor_paf = AnchorHit(chr(col["right_strand"][i]), col["rightscore"][i], col["righttstart"][i],
-                                              col["righttend"][i])
-            read.dist_between_anchors = col["dist_between_anchors"][i]
-            rr.read_dict[name] = read
-            rr.buffer_len = BUFFER_LEN
-            read.core_seq_start_pos, read.core_seq_end_pos = col["core_start"][i], col["core_end"][i]
-            read.mid_seq_start_pos, read.mid_seq_end_pos = col["mid_start"][i], col["mid_end"][i]
-            read.left_buffer_len, read.right_buffer_len = col["left_buffer"][i], col["right_buffer"][i]
-            read.strand = chr(col["strand"][i])
+        add_accepted_reads(rr, [names[i - first] for i in rows], col, rows, read_class)
         first = end
     return
+
+
+# The per-read Step-1 columns add_accepted_reads reads (strands as character codes), in the order
+# sharding.anchor_regions_sharded sends them between ranks.
+STEP1_FIELDS = ("read_len", "dist_between_anchors", "core_start", "core_end", "mid_start", "mid_end", "left_buffer",
+                "right_buffer", "strand", "left_strand", "right_strand", "leftscore", "lefttstart", "lefttend",
+                "rightscore", "righttstart", "righttend")
+
+
+def add_accepted_reads(repeat_region, names, col, rows, read_class=None):
+    """A Read per accepted read into repeat_region.read_dict, in the order given (:181-234): names[j] is the read whose
+    Step-1 fields are row rows[j] of the columns `col` ({STEP1_FIELDS name: sequence}).  A name given twice keeps its
+    first position in read_dict and the later read's fields, as the reference's dictionary does."""
+    if read_class is None:
+        from .repeat_region import Read as read_class
+    for name, i in zip(names, rows):
+        read = read_class()
+        read.read_name = name
+        read.full_read_len = col["read_len"][i]
+        read.left_anchor_is_good = read.right_anchor_is_good = read.both_anchors_are_good = True
+        read.left_anchor_paf = AnchorHit(chr(col["left_strand"][i]), col["leftscore"][i], col["lefttstart"][i], col["lefttend"][i])
+        read.right_anchor_paf = AnchorHit(chr(col["right_strand"][i]), col["rightscore"][i], col["righttstart"][i],
+                                          col["righttend"][i])
+        read.dist_between_anchors = col["dist_between_anchors"][i]
+        repeat_region.read_dict[name] = read
+        repeat_region.buffer_len = BUFFER_LEN
+        read.core_seq_start_pos, read.core_seq_end_pos = col["core_start"][i], col["core_end"][i]
+        read.mid_seq_start_pos, read.mid_seq_end_pos = col["mid_start"][i], col["mid_end"][i]
+        read.left_buffer_len, read.right_buffer_len = col["left_buffer"][i], col["right_buffer"][i]
+        read.strand = chr(col["strand"][i])
 
 
 def find_anchor_locations_in_reads(data_type, repeat_region, num_cpu=1, reads=None, read_class=None):

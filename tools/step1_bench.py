@@ -55,11 +55,11 @@ def shapes():
     loci = []
     for g in range(50):
         reg, _n, seqs, _t = synth.region_reads(seed=300 + g, n_reads=30, motif=("CAG", "GGGGCC", "AT", "TTTCA")[g % 4], alleles=(15, 45))
-        loci.append((reg.left_anchor_seq, reg.right_anchor_seq, seqs))
+        loci.append((reg.left_anchor_seq, reg.right_anchor_seq, seqs, reg.repeat_unit_seq))
     amp = []
     for g, motif in enumerate(("CAG", "CCG")):
         reg, _n, seqs, _t = synth.region_reads(seed=400 + g, n_reads=5000, motif=motif, alleles=(20, 40), outer=150)
-        amp.append((reg.left_anchor_seq, reg.right_anchor_seq, seqs))
+        amp.append((reg.left_anchor_seq, reg.right_anchor_seq, seqs, reg.repeat_unit_seq))
     return {"config1_15x30": loci[:15], "catalog_2000x30": [loci[g % 50] for g in range(2000)], "config2_2x5000": amp}
 
 
@@ -99,7 +99,7 @@ def main():
         res, stats = batched()
         # same accepted reads, strands, distances and cores as the per-region path
         i = 0
-        for (l, r, seqs) in regs[:200]:
+        for (l, r, seqs, _m) in regs[:200]:
             want = per_region(sc, l, r, seqs)
             got = {j: (chr(res[i + j]["strand"]), int(res[i + j]["dist_between_anchors"]), int(res[i + j]["core_start"]),
                        int(res[i + j]["core_end"])) for j in range(len(seqs)) if res[i + j]["accepted"]}
@@ -109,21 +109,21 @@ def main():
         for _ in range(args.reps):
             t0 = time.perf_counter(); batched(); t.append(time.perf_counter() - t0)
         e2e_new = sum(t) / len(t)
-        per_region(sc, *regs[0])
+        per_region(sc, *regs[0][:3])
         t0 = time.perf_counter()
-        for l, r, seqs in regs:
+        for l, r, seqs, _m in regs:
             per_region(sc, l, r, seqs)
         e2e_old = time.perf_counter() - t0
         k_new = kernel_ms(batched)
         k_old = kernel_ms(lambda: [engine.score_tasks([x for _s in seqs for x in (l, l, r, r)],
-                                                      [x for s in seqs for x in (s, rev_comp(s), s, rev_comp(s))], sc) for l, r, seqs in regs])
+                                                      [x for s in seqs for x in (s, rev_comp(s), s, rev_comp(s))], sc) for l, r, seqs, _m in regs])
         cells = stats["algorithmic_cells"]
         dev_new = sum(k_new.values())
         dev_old = sum(k_old.values())
         pair_ms = k_new.get("anchor_pair_kernel", 0.0)
         # cells the anchor kernel executes: both halves of 32 R S rows per read strand (nr_anchor.cu, pair_shape)
         rows = lambda n: (lambda S: S * 32 * next(h for h in (4, 6, 8, 12, 16) if h * 32 * S >= n))(max(1, -(-n // 512)))  # noqa: E731
-        pair_cells = sum(2 * 2 * rows(max(len(l), len(r))) * len(s) for l, r, seqs in regs for s in seqs)
+        pair_cells = sum(2 * 2 * rows(max(len(l), len(r))) * len(s) for l, r, seqs, _m in regs for s in seqs)
         doc["shapes"][name] = {
             "regions": len(regs), "reads": sum(map(len, reads)), "algorithmic_cells": cells, "stats": stats,
             "per_region": {"e2e_ms": e2e_old * 1e3, "device_ms": dev_old, "kernels_ms": k_old, "gcups_e2e": cells / e2e_old / 1e9,
