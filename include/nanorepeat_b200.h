@@ -306,6 +306,16 @@ int nr_anchor_regions(const nr_scoring_t* sc, int32_t n_regions, const nr_anchor
  * equal score the one with the highest window score is the alignment (the CPU checker under oracle/ states the same rule; its
  * traceback's CIGAR re-scored by the reference's own function gives the same number: tests/golden/make_golden_window.py).
  * A read is aligned as given and as its reverse complement when asked (the joint CLI feeds raw reads of either strand).
+ *
+ * Limits of the joint path (not nr_limits: the DP word here is score * 65536 + a signed 16-bit window score).  A task
+ * (nr_window_tasks) or grid point (nr_joint_grid) is not scored -- its record is (0, 0), the same as "no alignment" --
+ * and is counted in nr_last_stats' n_skipped when
+ *   - its template holds a base other than ACGT (reads may hold any character: it scores -ambiguous);
+ *   - match * min(|read|, |template|) > 32767 (reads longer than 16 383 bases are scored against shorter templates);
+ *   - its window is wider than 8 000 template bases (window scores up to +16 000 fit the 16-bit field);
+ *   - its template is longer than 2^20 bases.
+ * Windows are clamped to [0, |template|) before anything else.  nr_last_stats after either call: n_tasks = tasks or grid
+ * points, n_skipped = tasks (nr_window_tasks) or grid points, not strands (nr_joint_grid), kernel_launches.
  */
 typedef struct nr_window_t { int32_t score, window_score; } nr_window_t;
 /* n independent (query, target, window [a, b)) tasks; reverse (nullable): 1 = align the query's reverse complement. */
@@ -362,7 +372,8 @@ int nr_gmm1d_fit(const nr_gmm_params_t* p, int32_t n_problems, const int64_t* of
                  const int32_t* n_components, const int64_t* region_id, double* lower, int32_t* iters,
                  double* weights, double* means, double* variances);
 
-/* Counters of the last nr_score_tasks / nr_round2_region / nr_round3_region call on this thread. */
+/* Counters of the last nr_score_tasks / nr_round2_region / nr_round3_region / nr_window_tasks / nr_joint_grid call on
+ * this thread. */
 int nr_last_stats(nr_stats_t* out);
 
 #ifdef __cplusplus

@@ -1527,4 +1527,5 @@ void ambiguity(const char* s, int len, uint32_t* m) { ambiguity_plane(s, len, m)
 int alloc(void** p, size_t bytes, bool pinned) { return cached_alloc(p, bytes, pinned ? BUF_PIN : BUF_DEV); }
 void release(void* p, size_t bytes, bool pinned) { cached_free(p, bytes, pinned ? BUF_PIN : BUF_DEV); }
 int check(const nr_scoring_t* sc) { return check_scoring(sc); }
+void set_last_stats(const nr_stats_t& st) { g_last_stats = st; }
 }  // namespace nri

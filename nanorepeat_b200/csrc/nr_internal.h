@@ -17,4 +17,5 @@ void ambiguity(const char* s, int len, uint32_t* m);   // bit plane of the bases
 int alloc(void** p, size_t bytes, bool pinned);
 void release(void* p, size_t bytes, bool pinned);
 int check(const nr_scoring_t* sc);
+void set_last_stats(const nr_stats_t& st);       // what nr_last_stats reports on this thread
 }  // namespace nri

@@ -6,6 +6,7 @@
 
 #include <algorithm>
 #include <chrono>
+#include <climits>
 #include <cstdio>
 #include <cstdlib>
 #include <map>
@@ -42,16 +43,28 @@ struct SeqPool {
     }
 };
 
+// The joint path's limits (include/nanorepeat_b200.h): the DP word holds score * 65536 + payload, so the score must stay
+// within 15 bits and the window within 8 000 bases (payload <= +16 000); the per-warp scratch row holds one template.
 constexpr int kMaxScore = 32767, kMaxWindow = 8000, kMaxTlen = 1 << 20;
 
-// tasks[i].q_word / t_word index `pool`; out[i] = (score, window score); skipped tasks (outside the packed range) stay 0
-int run_window_tasks(const nr_scoring_t* sc, std::vector<nrw::WinTask>& tasks, const SeqPool& pool, nr_window_t* out, int* n_skipped) {
+// Every pool word a kernel reads through a 32-bit task field must fit it.
+int check_pool(const SeqPool& pool, const char* who) {
+    if (pool.words.size() + 4 > (size_t)UINT32_MAX) return nri::fail_msg(NR_ERR_ARG, who);
+    return NR_OK;
+}
+
+// tasks[i].q_word / t_word index `pool`; out[i] = (score, window score).  skipped[i] (in: 1 for a template the pool could
+// not pack) is set for every task beyond the limits above; a skipped task is not scored and its record stays (0, 0).
+int run_window_tasks(const nr_scoring_t* sc, std::vector<nrw::WinTask>& tasks, const SeqPool& pool, nr_window_t* out,
+                     std::vector<uint8_t>& skipped, int& launches) {
     const int n = (int)tasks.size();
     if (n == 0) return NR_OK;
+    if (int rc = check_pool(pool, "joint path: more than 2^32 words of packed sequence in one call")) return rc;
     int max_t = 1;
-    for (nrw::WinTask& t : tasks) {
+    for (int i = 0; i < n; ++i) {
+        nrw::WinTask& t = tasks[i];
         const long long m = (long long)sc->match * std::min(t.q_len, t.t_len);
-        if (m > kMaxScore || t.win_b - t.win_a > kMaxWindow || t.t_len > kMaxTlen) { t.q_len = 0; if (n_skipped) ++*n_skipped; }
+        if (m > kMaxScore || t.win_b - t.win_a > kMaxWindow || t.t_len > kMaxTlen) { t.q_len = 0; skipped[i] = 1; }
         max_t = std::max(max_t, t.t_len);
     }
     // long tasks first: the tail of the launch is made of short ones
@@ -94,6 +107,7 @@ int run_window_tasks(const nr_scoring_t* sc, std::vector<nrw::WinTask>& tasks, c
                                                                   static_cast<int4*>(d_scratch), stride, static_cast<int*>(d_counter),
                                                                   static_cast<int2*>(d_out));
         e = cudaGetLastError();
+        ++launches;
     }
     if (e == cudaSuccess) e = cudaMemcpyAsync(h_out, d_out, out_bytes, cudaMemcpyDeviceToHost, st);
     const auto t_launch = std::chrono::steady_clock::now();
@@ -132,7 +146,7 @@ nrw::WinScore window_score_words(const nr_scoring_t* sc) {
 // The shared-sweep path (nr_window_ladder.cuh): backward tasks, then forward tasks; res[out_off + j] of every forward task.
 int run_ladder_tasks(const nr_scoring_t* sc, const std::vector<nrw::LadBwdTask>& btasks, std::vector<nrw::LadFwdTask>& ptasks,
                      std::vector<nrw::LadFwdTask>& ftasks, const SeqPool& pool, size_t bvec_words, size_t cstate_words, size_t n_pbest1,
-                     size_t n_out, int max_t, std::vector<int2>& res) {
+                     size_t n_out, int max_t, std::vector<int2>& res, int& launches) {
     const int nb = (int)btasks.size(), nf = (int)ftasks.size(), np = (int)ptasks.size();
     res.assign(n_out, make_int2(0, 0));
     if (nf == 0) return NR_OK;
@@ -185,6 +199,7 @@ int run_ladder_tasks(const nr_scoring_t* sc, const std::vector<nrw::LadBwdTask>&
                                                                      static_cast<const uint32_t*>(d_pool), k, static_cast<int4*>(d_scratch),
                                                                      stride, counter, static_cast<int*>(d_bvec), static_cast<int*>(d_ronly));
     JTRY(cudaGetLastError());
+    ++launches;
     if (np) {       // prefix sweeps: the columns the continuation sweeps start from
         nrw::ladder_fwd_kernel<<<blocks_p, 32 * nrw::kWarps, smem_f, st>>>(static_cast<const nrw::LadFwdTask*>(d_p), np,
                                                                          static_cast<const nrw::LadBwdTask*>(d_b), static_cast<const uint32_t*>(d_pool),
@@ -193,6 +208,7 @@ int run_ladder_tasks(const nr_scoring_t* sc, const std::vector<nrw::LadBwdTask>&
                                                                          static_cast<int*>(d_cstate), static_cast<int*>(d_pbest1),
                                                                          static_cast<int2*>(d_out));
         JTRY(cudaGetLastError());
+        ++launches;
     }
     nrw::ladder_fwd_kernel<<<blocks_f, 32 * nrw::kWarps, smem_f, st>>>(static_cast<const nrw::LadFwdTask*>(d_f), nf,
                                                                      static_cast<const nrw::LadBwdTask*>(d_b), static_cast<const uint32_t*>(d_pool),
@@ -201,6 +217,7 @@ int run_ladder_tasks(const nr_scoring_t* sc, const std::vector<nrw::LadBwdTask>&
                                                                      static_cast<int*>(d_cstate), static_cast<int*>(d_pbest1),
                                                                      static_cast<int2*>(d_out));
     JTRY(cudaGetLastError());
+    ++launches;
     JTRY(cudaMemcpyAsync(h_out, d_out, out_bytes, cudaMemcpyDeviceToHost, st));
     const auto t_launch = std::chrono::steady_clock::now();
     const cudaError_t e = cudaStreamSynchronize(st);
@@ -222,8 +239,12 @@ extern "C" int nr_window_tasks(const nr_scoring_t* sc, int32_t n_tasks, const ch
         return nri::fail_msg(NR_ERR_ARG, "nr_window_tasks: bad arguments");
     int rc = nri::ensure_init();
     if (rc) return rc;
+    nr_stats_t st = {};
+    st.n_tasks = n_tasks;
+    nri::set_last_stats(st);
     SeqPool pool;
     std::vector<nrw::WinTask> tasks(n_tasks);
+    std::vector<uint8_t> skipped(n_tasks, 0);
     std::map<std::pair<const char*, int>, long long> seen_q, seen_t;
     for (int i = 0; i < n_tasks; ++i) {
         nrw::WinTask& t = tasks[i];
@@ -237,10 +258,16 @@ extern "C" int nr_window_tasks(const nr_scoring_t* sc, int32_t n_tasks, const ch
         const long long tw = seen_t[tk];
         t.q_word = (uint32_t)seen_q[qk]; t.q_len = qlen[i];
         t.t_word = tw < 0 ? 0u : (uint32_t)tw; t.t_len = tw < 0 ? 0 : tlen[i];      // a template with N is not scored
+        skipped[i] = tw < 0;
         t.win_a = std::max(0, win_a[i]); t.win_b = std::min(win_b[i], tlen[i]);
         t.reverse = reverse ? reverse[i] != 0 : 0;
     }
-    return run_window_tasks(sc, tasks, pool, out, nullptr);
+    int launches = 0;
+    rc = run_window_tasks(sc, tasks, pool, out, skipped, launches);
+    st.kernel_launches = launches;
+    for (uint8_t k : skipped) st.n_skipped += k;
+    nri::set_last_stats(st);
+    return rc;
 }
 
 extern "C" int nr_joint_grid(const nr_scoring_t* sc, const char* left, int32_t n_left, const char* mid, int32_t n_mid,
@@ -255,6 +282,10 @@ extern "C" int nr_joint_grid(const nr_scoring_t* sc, const char* left, int32_t n
         return nri::fail_msg(NR_ERR_ARG, "nr_joint_grid: bad arguments");
     int rc = nri::ensure_init();
     if (rc) return rc;
+    nr_stats_t st = {};
+    st.n_tasks = n_points;
+    nri::set_last_stats(st);
+    int launches = 0;
     const bool tracing = getenv("NR_TRACE") != nullptr;
     auto t_mark = std::chrono::steady_clock::now();
     auto mark = [&](const char* what) {
@@ -373,7 +404,7 @@ extern "C" int nr_joint_grid(const nr_scoring_t* sc, const char* left, int32_t n
                 nrw::LadBwdTask bt = {};
                 bt.q_word = (uint32_t)read_word[r]; bt.q_len = read_len[r];
                 bt.rev_word = (uint32_t)rev_word; bt.n_right = n_right;
-                bt.reverse = sd; bt.bvec_off = (int)bvec_words;
+                bt.reverse = sd; bt.set_bvec_off((long long)bvec_words);
                 bvec_words += 3 * (size_t)read_len[r];
                 btasks.push_back(bt);
             }
@@ -425,8 +456,14 @@ extern "C" int nr_joint_grid(const nr_scoring_t* sc, const char* left, int32_t n
     }
     mark("tasks of the shared sweeps");
     if (!ftasks.empty()) {
+        // out_off, pbest1 and bwd are 32-bit task fields (bvec_off and cstate are 64-bit)
+        if (n_lad_out > (size_t)INT_MAX || n_pbest1 > (size_t)INT_MAX || btasks.size() > (size_t)INT_MAX ||
+            ftasks.size() > (size_t)INT_MAX)
+            return nri::fail_msg(NR_ERR_ARG, "nr_joint_grid: more than 2^31 records of the shared sweeps in one call");
+        if ((rc = check_pool(pool, "nr_joint_grid: more than 2^32 words of packed sequence in one call"))) return rc;
         std::vector<int2> res;
-        if ((rc = run_ladder_tasks(sc, btasks, ptasks, ftasks, pool, bvec_words, cstate_words, n_pbest1, n_lad_out, lad_max_t, res))) return rc;
+        if ((rc = run_ladder_tasks(sc, btasks, ptasks, ftasks, pool, bvec_words, cstate_words, n_pbest1, n_lad_out, lad_max_t, res, launches)))
+            return rc;
         for (int i = 0; i < n_points; ++i) {
             if (!by_ladder[i]) continue;
             const int2 f = res[point_slot[i]], v = res[point_slot_rev[i]];
@@ -442,6 +479,7 @@ extern "C" int nr_joint_grid(const nr_scoring_t* sc, const char* left, int32_t n
     std::map<std::pair<int, int>, std::pair<long long, int>> tpl;      // (k1, k2) -> (word, length)
     std::vector<nrw::WinTask> tasks;
     std::vector<int> task_point;
+    std::vector<uint8_t> no_tpl;                                      // per grid point: its template holds a base other than ACGT
     std::string s;
     for (int i = 0; i < n_points; ++i) {
         if (by_ladder[i]) continue;
@@ -466,16 +504,22 @@ extern "C" int nr_joint_grid(const nr_scoring_t* sc, const char* left, int32_t n
         t.reverse = 0; tasks.push_back(t);
         t.reverse = 1; tasks.push_back(t);
         task_point.push_back(i);
+        no_tpl.push_back(tw < 0);
     }
     std::vector<nr_window_t> res(tasks.size());
-    if ((rc = run_window_tasks(sc, tasks, pool, res.data(), nullptr))) return rc;
+    std::vector<uint8_t> skipped(tasks.size(), 0);
+    for (size_t j = 0; j < tasks.size(); ++j) skipped[j] = no_tpl[j / 2];
+    if ((rc = run_window_tasks(sc, tasks, pool, res.data(), skipped, launches))) return rc;
+    st.kernel_launches = launches;
     for (size_t j = 0; j < task_point.size(); ++j) {
         const int i = task_point[j];
+        st.n_skipped += skipped[2 * j] | skipped[2 * j + 1];                       // once per grid point
         const nr_window_t f = res[2 * j], v = res[2 * j + 1];
         // the better strand by (score, window score); '+' on a full tie
         const bool rev = v.score > f.score || (v.score == f.score && v.window_score > f.window_score);
         out[i] = rev ? v : f;
         if (strand) strand[i] = rev ? 1 : 0;
     }
+    nri::set_last_stats(st);
     return NR_OK;
 }

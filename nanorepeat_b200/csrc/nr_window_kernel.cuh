@@ -16,8 +16,11 @@
 //   insertion step at template position p:        -4 if it opens the run, else -2, if a < p < b - 1
 // Integer max on words is the lexicographic max of (score, payload): among all optimal alignments the canonical one is
 // the one with the highest window score (the CPU checker under oracle/ has the same rule and a traceback; the
-// golden vectors run the reference's own CIGAR re-scoring on the traceback's CIGAR).  Score range: payload stays
-// within +-32767 for windows up to 8 000 template bases, scores up to 32 767.
+// golden vectors run the reference's own CIGAR re-scoring on the traceback's CIGAR).  Score range: the payload decodes
+// as a signed 16-bit value.  Its ceiling is +2 per window base, +16 000 at the 8 000-base window limit.  Its floor is an
+// insertion charged in full, bounded by the score limit (match * min(q, t) <= 32 767): a 16 356-base insertion into a
+// 3-base window of a 16 383-base template gives (16 386, -32 708), 60 from the decode limit at the score limit
+// (tests/test_gpu_joint_edges.py).
 //
 // Mapping: one warp per (read, template) task, 8 rows per lane, the read cut into stripes of 256 rows that the SAME warp
 // sweeps one after the other; the bottom row of a stripe (H, F1, F2 per template column) travels through a per-warp

@@ -41,9 +41,15 @@ struct LadBwdTask {        // one per (read, strand)
     uint32_t q_word; int32_t q_len;
     uint32_t rev_word; int32_t n_right;    // reverse(right)
     int32_t reverse;                       // strand
-    int32_t bvec_off;                      // first word of this task's junction vectors: 3 planes of q_len words
-    int32_t pad[2];
+    int32_t pad;
+    // First word of this task's junction vectors (3 planes of q_len words).  64-bit: a call spends 6 words per read base
+    // on the shared path, past 2^31 after ~358 M bases.  Kept as two 32-bit halves: a long long member makes the struct
+    // 8-byte aligned, and ptxas then gives both ladder kernels 128 registers (64 / 80 with the halves) and a spill.
+    uint32_t bvec_lo, bvec_hi;
+    __host__ __device__ long long bvec_off() const { return (long long)(((unsigned long long)bvec_hi << 32) | bvec_lo); }
+    void set_bvec_off(long long w) { bvec_lo = (uint32_t)w; bvec_hi = (uint32_t)((unsigned long long)w >> 32); }
 };
+static_assert(sizeof(LadBwdTask) == 32, "LadBwdTask is 32 bytes");
 
 struct LadFwdTask {        // one per (read, strand, k1)
     uint32_t q_word; int32_t q_len;
@@ -341,7 +347,7 @@ ladder_bwd_kernel(const LadBwdTask* __restrict__ tasks, int n_tasks, const uint3
         i = __shfl_sync(kFull, i, 0);
         if (i >= n_tasks) break;
         const LadBwdTask tk = tasks[i];
-        ladder_bwd_task(tk, pool, sc, prof, bnd, bvec + tk.bvec_off, ronly + i, lane);
+        ladder_bwd_task(tk, pool, sc, prof, bnd, bvec + tk.bvec_off(), ronly + i, lane);
     }
 }
 
@@ -366,9 +372,9 @@ ladder_fwd_kernel(const LadFwdTask* __restrict__ tasks, int n_tasks, const LadBw
         if (tk.mode == kPrefix)
             ladder_fwd_task<kPrefix>(tk, pool, sc, prof, bsm, jbest, pbest, bnd, bvec, 0, cstate, pbest1, out, lane);
         else if (tk.mode == kCont)
-            ladder_fwd_task<kCont>(tk, pool, sc, prof, bsm, jbest, pbest, bnd, bvec + btasks[tk.bwd].bvec_off, ronly[tk.bwd], cstate, pbest1, out, lane);
+            ladder_fwd_task<kCont>(tk, pool, sc, prof, bsm, jbest, pbest, bnd, bvec + btasks[tk.bwd].bvec_off(), ronly[tk.bwd], cstate, pbest1, out, lane);
         else
-            ladder_fwd_task<kWhole>(tk, pool, sc, prof, bsm, jbest, pbest, bnd, bvec + btasks[tk.bwd].bvec_off, ronly[tk.bwd], cstate, pbest1, out, lane);
+            ladder_fwd_task<kWhole>(tk, pool, sc, prof, bsm, jbest, pbest, bnd, bvec + btasks[tk.bwd].bvec_off(), ronly[tk.bwd], cstate, pbest1, out, lane);
     }
 }
 
