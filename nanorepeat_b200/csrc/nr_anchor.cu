@@ -15,7 +15,6 @@
 //      hold the score (match * min(|anchor|, |read|) > 32767) the anchor gets no hit on that read and n_skipped counts it.
 // Then the reference's rules, on the host.
 #include "nr_batch.h"
-#include "nr_internal.h"
 #include "nr_launch_anchor.h"
 
 #include <algorithm>
@@ -26,32 +25,8 @@
 
 namespace {
 
-#define ATRY(expr)                                                                                       \
-    do {                                                                                                 \
-        cudaError_t e__ = (expr);                                                                        \
-        if (e__ != cudaSuccess) {                                                                        \
-            char b__[512];                                                                               \
-            snprintf(b__, sizeof b__, "%s failed: %s (%s:%d)", #expr, cudaGetErrorString(e__), __FILE__, __LINE__); \
-            cudaGetLastError();                                                                          \
-            return nri::fail_msg(NR_ERR_CUDA, b__);                                                      \
-        }                                                                                                \
-    } while (0)
-
 constexpr int kMaxPairAnchor = (65535 - 65) / 4;   // a half holds 2 * score + 65 and score <= 2 * |anchor| (map-ont)
 constexpr int kBufferLen = 100;                    // nanoRepeat_bam.py:221
-
-// Device and pinned buffers of one call, given back to the caching allocator on scope exit.
-struct Bufs {
-    struct One { void* p; size_t bytes; bool pinned; };
-    std::vector<One> all;
-    int get(void** p, size_t bytes, bool pinned) {
-        *p = nullptr;
-        const int rc = nri::alloc(p, bytes, pinned);
-        if (rc == NR_OK) all.push_back({*p, bytes, pinned});
-        return rc;
-    }
-    ~Bufs() { for (const One& b : all) nri::release(b.p, b.bytes, b.pinned); }
-};
 
 inline char complement(char c) {
     switch (c) {
@@ -80,7 +55,7 @@ int anchor_regions(const nr_scoring_t* sc, int n_regions, const nr_anchor_region
         const nr_anchor_region_t& G = regs[g];
         if (G.n_reads < 0 || G.n_left < 0 || G.n_right < 0 || G.reads_len < 0 || (G.n_left > 0 && !G.left) ||
             (G.n_right > 0 && !G.right) || (G.n_reads > 0 && !G.reads))
-            return nri::fail_msg(NR_ERR_ARG, "nr_anchor_regions: a region has bad arguments");
+            return nri::fail(NR_ERR_ARG, "nr_anchor_regions: a region has bad arguments");
         first[g + 1] = first[g] + G.n_reads;
     }
     const long long total = first[n_regions];
@@ -92,11 +67,8 @@ int anchor_regions(const nr_scoring_t* sc, int n_regions, const nr_anchor_region
         for (int i = 0; i < G.n_reads; ++i) {
             const char* nl = pos < G.reads_len ? static_cast<const char*>(memchr(G.reads + pos, '\n', (size_t)(G.reads_len - pos))) : nullptr;
             const long long end = nl ? nl - G.reads : G.reads_len;
-            if ((!nl && i + 1 < G.n_reads) || (nl && i + 1 == G.n_reads) || end - pos > 0x7fffffffLL) {
-                char b[160];
-                snprintf(b, sizeof b, "nr_anchor_regions: region %d does not hold %d lines (a read holds a newline?)", g, G.n_reads);
-                return nri::fail_msg(NR_ERR_BAD_BASE, b);
-            }
+            if ((!nl && i + 1 < G.n_reads) || (nl && i + 1 == G.n_reads) || end - pos > 0x7fffffffLL)
+                return nri::fail(NR_ERR_BAD_BASE, "nr_anchor_regions: region %d does not hold %d lines (a read holds a newline?)", g, G.n_reads);
             rptr[r + i] = G.reads + pos;
             rlen[r + i] = (int)(end - pos);
             pos = end + 1;
@@ -105,7 +77,7 @@ int anchor_regions(const nr_scoring_t* sc, int n_regions, const nr_anchor_region
     int rc = nri::ensure_init();
     if (rc) return rc;
     nr_stats_t st = {};
-    nrh::Pool pool;        // anchors are queries (an ambiguity plane for bases other than ACGT), read strands templates
+    nri::Pool pool;        // anchors are queries (an ambiguity plane for bases other than ACGT), read strands templates
     {
         size_t words = 0;
         for (long long i = 0; i < total; ++i) words += 2 * ((size_t)(rlen[i] + 15) / 16 + 1);
@@ -130,7 +102,7 @@ int anchor_regions(const nr_scoring_t* sc, int n_regions, const nr_anchor_region
         for (int j = 0; j < rlen[i]; ++j) s[j] = complement(rptr[i][rlen[i] - 1 - j]);
         rev_word[i] = pool.add(s.data(), rlen[i], false);
     }
-    if (pool.words.size() > 0xfffffff0ULL) return nri::fail_msg(NR_ERR_TOO_LARGE, "nr_anchor_regions: sequence pool exceeds 2^32 words");
+    if (pool.words.size() > 0xfffffff0ULL) return nri::fail(NR_ERR_TOO_LARGE, "nr_anchor_regions: sequence pool exceeds 2^32 words");
 
     // cand[(4 * read + 2 * anchor + strand)]: anchor 0 left, 1 right; strand 0 '+', 1 '-'
     std::vector<Cand> cand(4 * (size_t)total);
@@ -171,7 +143,7 @@ int anchor_regions(const nr_scoring_t* sc, int n_regions, const nr_anchor_region
         const size_t pair_bytes = sizeof(nr::pr::AnchorPair) * n_pairs, pool_bytes = sizeof(uint32_t) * (pool.words.size() + 4),
                      key_bytes = sizeof(uint2) * n_pairs,
                      scratch_bytes = sizeof(ulonglong2) * 2 * stride * (size_t)blocks * nr::kWarpsPerBlock;
-        Bufs bufs;
+        nri::Bufs bufs;
         void *h_in = nullptr, *d_in = nullptr, *d_keys = nullptr, *h_keys = nullptr, *d_scratch = nullptr, *d_counter = nullptr;
         if ((rc = bufs.get(&h_in, pair_bytes + pool_bytes, true)) || (rc = bufs.get(&d_in, pair_bytes + pool_bytes, false)) ||
             (rc = bufs.get(&d_keys, key_bytes, false)) || (rc = bufs.get(&h_keys, key_bytes, true)) ||
@@ -180,17 +152,17 @@ int anchor_regions(const nr_scoring_t* sc, int n_regions, const nr_anchor_region
         memcpy(h_in, order.data(), pair_bytes);
         memcpy(static_cast<char*>(h_in) + pair_bytes, pool.words.data(), sizeof(uint32_t) * pool.words.size());
         cudaStream_t s = nri::stream();
-        ATRY(cudaMemcpyAsync(d_in, h_in, pair_bytes + pool_bytes, cudaMemcpyHostToDevice, s));
-        ATRY(cudaMemsetAsync(d_counter, 0, 256, s));
+        CUDA_TRY(cudaMemcpyAsync(d_in, h_in, pair_bytes + pool_bytes, cudaMemcpyHostToDevice, s));
+        CUDA_TRY(cudaMemsetAsync(d_counter, 0, 256, s));
         int* counter = static_cast<int*>(d_counter);
-        ATRY(nrl::launch_anchor_pairs(blocks, s, static_cast<const nr::pr::AnchorPair*>(d_in), n_pairs,
+        CUDA_TRY(nrl::launch_anchor_pairs(blocks, s, static_cast<const nr::pr::AnchorPair*>(d_in), n_pairs,
                                       reinterpret_cast<const uint32_t*>(static_cast<char*>(d_in) + pair_bytes),
                                       static_cast<ulonglong2*>(d_scratch), stride, counter, static_cast<uint2*>(d_keys)));
-        ATRY(cudaMemcpyAsync(h_keys, d_keys, key_bytes, cudaMemcpyDeviceToHost, s));
+        CUDA_TRY(cudaMemcpyAsync(h_keys, d_keys, key_bytes, cudaMemcpyDeviceToHost, s));
         int spin = 0;
-        ATRY(cudaMemcpyAsync(&spin, counter + 1, sizeof(int), cudaMemcpyDeviceToHost, s));
-        ATRY(cudaStreamSynchronize(s));
-        if (spin) return nri::fail_msg(NR_ERR_CUDA, "nr_anchor_regions: a stripe gave up waiting for the stripe above it");
+        CUDA_TRY(cudaMemcpyAsync(&spin, counter + 1, sizeof(int), cudaMemcpyDeviceToHost, s));
+        CUDA_TRY(cudaStreamSynchronize(s));
+        if (spin) return nri::fail(NR_ERR_CUDA, "nr_anchor_regions: a stripe gave up waiting for the stripe above it");
         ++st.kernel_launches;
         st.n_tasks += n_pairs;
         st.h2d_bytes += (int64_t)(pair_bytes + pool_bytes);
@@ -243,7 +215,7 @@ int anchor_regions(const nr_scoring_t* sc, int n_regions, const nr_anchor_region
             for (long long i = first[g]; i < first[g + 1]; ++i) {
                 if (fwd_word[i] < 0 || n == 0) continue;
                 if (n > kMaxPairAnchor) {
-                    if ((long long)sc->match * std::min(n, rlen[i]) > nrh::kMaxScore) {     // no DP word holds its score:
+                    if ((long long)sc->match * std::min(n, rlen[i]) > nri::kMaxScore) {     // no DP word holds its score:
                         ++st.n_skipped;                                                     // no hit, counted once
                         continue;
                     }
@@ -285,12 +257,9 @@ int anchor_regions(const nr_scoring_t* sc, int n_regions, const nr_anchor_region
                 c.score = res[t].score; c.tstart = res[t].tstart; c.tend = res[t].tend;
                 continue;
             }
-            if (res[t].score != c.score || res[t].tend != c.tend - twin[t]) {
-                char m[200];
-                snprintf(m, sizeof m, "nr_anchor_regions: start recovery of a hit (%d, end %d) found (%d, %d, %d) in its window",
-                         c.score, c.tend, res[t].score, twin[t] + res[t].tstart, twin[t] + res[t].tend);
-                return nri::fail_msg(NR_ERR_CUDA, m);
-            }
+            if (res[t].score != c.score || res[t].tend != c.tend - twin[t])
+                return nri::fail(NR_ERR_CUDA, "nr_anchor_regions: start recovery of a hit (%d, end %d) found (%d, %d, %d) in its window",
+                                 c.score, c.tend, res[t].score, twin[t] + res[t].tstart, twin[t] + res[t].tend);
             c.tstart = twin[t] + res[t].tstart;
         }
     }
@@ -338,11 +307,11 @@ int anchor_regions(const nr_scoring_t* sc, int n_regions, const nr_anchor_region
 extern "C" int nr_anchor_regions(const nr_scoring_t* sc, int32_t n_regions, const nr_anchor_region_t* regions, nr_anchor_read_t* out,
                                  nr_stats_t* stats) {
     if (nri::check(sc)) return nri::last_code();
-    if (n_regions < 0 || (n_regions > 0 && !regions)) return nri::fail_msg(NR_ERR_ARG, "nr_anchor_regions: bad arguments");
+    if (n_regions < 0 || (n_regions > 0 && !regions)) return nri::fail(NR_ERR_ARG, "nr_anchor_regions: bad arguments");
     if (!nrh::is_map_ont(*sc) || sc->min_dp_score < 10 * sc->match)
-        return nri::fail_msg(NR_ERR_ARG, "nr_anchor_regions: needs map-ont scoring with min_dp_score >= 10 * match");
+        return nri::fail(NR_ERR_ARG, "nr_anchor_regions: needs map-ont scoring with min_dp_score >= 10 * match");
     long long total = 0;
     for (int g = 0; g < n_regions; ++g) total += std::max(0, regions[g].n_reads);
-    if (total > 0 && !out) return nri::fail_msg(NR_ERR_ARG, "nr_anchor_regions: out is NULL");
+    if (total > 0 && !out) return nri::fail(NR_ERR_ARG, "nr_anchor_regions: out is NULL");
     return anchor_regions(sc, n_regions, regions, out, stats);
 }

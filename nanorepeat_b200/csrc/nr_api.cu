@@ -26,6 +26,7 @@
 #include <vector>
 
 using namespace nrh;
+using nri::fail;
 
 namespace {
 
@@ -35,7 +36,7 @@ thread_local nr_stats_t g_last_stats = {};
 
 }  // namespace
 
-int nrh::fail(int code, const char* fmt, ...) {
+int nri::fail(int code, const char* fmt, ...) {
     char buf[512];
     va_list ap;
     va_start(ap, fmt);
@@ -47,14 +48,6 @@ int nrh::fail(int code, const char* fmt, ...) {
 }
 
 namespace {
-
-#define CUDA_TRY(expr)                                                                          \
-    do {                                                                                        \
-        cudaError_t e__ = (expr);                                                               \
-        if (e__ != cudaSuccess)                                                                 \
-            return fail(NR_ERR_CUDA, "%s failed: %s (%s:%d)", #expr, cudaGetErrorString(e__),   \
-                        __FILE__, __LINE__);                                                    \
-    } while (0)
 
 using nr::kWarpsPerBlock;
 
@@ -296,7 +289,7 @@ nr::ScoreW score_words(const nr_scoring_t& sc) {
 // Allocates the buffers plan_batch sized, stages the blob's sections in pinned memory and uploads them on the library's
 // stream (asynchronously: nr_batch_run orders itself behind ev_uploaded).
 int upload_batch(nr_batch* b) {
-    PhaseTrace trace;
+    nri::PhaseTrace trace;
     int rc;
     if ((rc = cached_alloc(&b->d_blob, b->blob_bytes, BUF_DEV))) return rc;
     if ((rc = cached_alloc(&b->h_blob, b->blob_bytes, BUF_PIN))) return rc;
@@ -880,7 +873,7 @@ int nr_set_ladder_mode(int mode) {
 }
 
 int nr_limits(int32_t* max_score, int32_t* max_tlen) {
-    if (max_score) *max_score = kMaxScore;
+    if (max_score) *max_score = nri::kMaxScore;
     if (max_tlen) *max_tlen = kMaxTlen;
     return NR_OK;
 }
@@ -1341,7 +1334,7 @@ int estimate_regions(const nr_scoring_t* sc, int fast_mode, int n_regions, const
     };
     if (stats) *stats = {};
     const int min_score = std::max(1, sc->min_dp_score);
-    PhaseTrace trace;
+    nri::PhaseTrace trace;
     trace.mark("estimate: round 1, grouping");
     // round 2 of every group (was pymm2.main at :362).  The reads of the groups are packed side by side on host threads
     // (pure CPU work on each group's own batch; batches are created here, on the thread that owns the CUDA context),
@@ -1515,12 +1508,11 @@ extern "C" int nr_estimate_regions(const nr_scoring_t* sc, int32_t fast_mode, in
     return estimate_regions(sc, fast_mode, n_regions, regions, r1, r2, r2_valid, r3, r3_state, T_out, stats);
 }
 
-// ---- what the other host translation units (nr_joint.cu, nr_anchor.cu) share with this one ----------------------------
+// ---- what the other host translation units share with this one (declared in nr_internal.h) ---------------------------
 namespace nri {
 int ensure_init() { return ::ensure_init(-1); }
 cudaStream_t stream() { return g_ctx.stream; }
 int sm_count() { return g_ctx.sm_count; }
-int fail_msg(int code, const char* msg) { return fail(code, "%s", msg); }
 int last_code() { return g_code; }
 bool pack(const char* s, int len, uint32_t* w) { return pack_seq(s, len, w); }
 void ambiguity(const char* s, int len, uint32_t* m) { ambiguity_plane(s, len, m); }

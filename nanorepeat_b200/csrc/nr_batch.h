@@ -1,50 +1,17 @@
-// nr_batch.h -- the batch behind the C ABI's nr_batch_t and the host services its planner (nr_plan.cu) shares with
-// nr_api.cu and nr_anchor.cu.  Host-only translation units include it; kernel translation units must not (their code
-// placement follows the exact text they are compiled from, DESIGN.md sections 4.10 and 9).
+// nr_batch.h -- the batch behind the C ABI's nr_batch_t and its planner (nr_plan.cu), shared by nr_api.cu and
+// nr_anchor.cu.  Host-only translation units include it; no kernel translation unit includes a host header: every kernel
+// family has a launcher unit of its own (nr_launch_*.cu), whose code placement follows the exact text it is compiled
+// from (DESIGN.md sections 4.10 and 9).
 #pragma once
 #include "nr_internal.h"
 #include "nr_launch.h"
 
-#include <chrono>
-#include <cmath>
-#include <cstdio>
-#include <cstdlib>
-#include <functional>
 #include <string>
-#include <thread>
 #include <vector>
 
 namespace nrh {
 
-constexpr int kMaxScore = 32767;   // signed 16-bit score field of the packed DP word
 constexpr int kMaxTlen = 65535 - 64; // unsigned 16-bit span field, minus the wavefront skew (step counters share it)
-
-int fail(int code, const char* fmt, ...);     // records the thread's last error (nr_last_error), returns code
-
-// Sequence pool.  Every sequence starts on a word boundary and is followed by one slack word (kernels prefetch one word
-// ahead).  For a READ the slack word doubles as the link to its ambiguity plane: 0 = ACGT only, otherwise the plane
-// starts that many words behind the read's first word (nr_kernels.cuh, read_has_ambiguous).  Templates must be ACGT.
-struct Pool {
-    std::vector<uint32_t> words;
-    // append; returns first word index, or -1 on a non-ACGT character (ambiguous_ok: append the plane instead)
-    long long add(const char* s, int len, bool ambiguous_ok = false) {
-        const size_t w0 = words.size();
-        const size_t nw = (size_t)(len + 15) / 16 + 1;
-        words.resize(w0 + nw, 0u);
-        if (!nri::pack(s, len, words.data() + w0)) {
-            if (!ambiguous_ok) { words.resize(w0); return -1; }
-            link_plane(w0, s, len);
-        }
-        return (long long)w0;
-    }
-    // append the ambiguity plane of the read packed at word w0 and link it from the read's slack word
-    void link_plane(size_t w0, const char* s, int len) {
-        const size_t at = words.size();
-        words.resize(at + (size_t)(len + 31) / 32, 0u);
-        nri::ambiguity(s, len, words.data() + at);
-        words[w0 + (size_t)(len + 15) / 16] = (uint32_t)(at - w0);
-    }
-};
 
 struct Launch {      // one persistent launch per batch
     bool ladder;     // ladder_kernel over nr_batch::ltasks instead of exact_kernel over nr_batch::tasks
@@ -81,20 +48,6 @@ inline bool is_map_ont(const nr_scoring_t& c) {
     return c.match == 2 && c.mismatch == 4 && c.gap_open1 == 4 && c.gap_ext1 == 2 && c.gap_open2 == 24 && c.gap_ext2 == 1 &&
            c.ambiguous == 1;
 }
-
-// NR_TRACE=1: host-side phase times of a commit on stderr (where a commit's half millisecond goes)
-struct PhaseTrace {
-    const bool on = getenv("NR_TRACE") != nullptr;
-    std::chrono::steady_clock::time_point t0 = std::chrono::steady_clock::now();
-    void mark(const char* what) {
-        if (!on) return;
-        const auto t1 = std::chrono::steady_clock::now();
-        fprintf(stderr, "[nr trace] %-28s %8.1f us   (ends at %10.1f us, thread %04x)\n", what,
-                std::chrono::duration<double, std::micro>(t1 - t0).count(), std::fmod(std::chrono::duration<double, std::micro>(t1.time_since_epoch()).count(), 1e8),
-                (unsigned)(std::hash<std::thread::id>()(std::this_thread::get_id()) & 0xffff));
-        t0 = t1;
-    }
-};
 
 }  // namespace nrh
 
@@ -139,7 +92,7 @@ struct nr_batch {
     int* d_flags = nullptr;                   // progress flags of the multi-stripe tasks, zeroed before every run
     size_t flags_bytes = 0;
     nrh::Launch launch = {};
-    nrh::Pool pool;
+    nri::Pool pool;
     // per-read bookkeeping (rounds 2 and 3)
     std::vector<nrh::RegionInfo> regions;
     int n_reads = 0;

@@ -1,255 +1,26 @@
 // nr_gmm.cu -- batched 1-D Gaussian-mixture phasing (SURVEY.md 8(f) row f3): what the reference does per region after
 // round 3 (nanoRepeat_bam.py:515-575, split_alleles.py:82-200) -- 3-sigma trim, 100x bootstrap with Gaussian noise
 // sd = error_rate * (10 + size), GaussianMixture(n, 'diag', n_init = 10) for n = 2, 3, ... until two components'
-// [isf(1 - o), isf(o)] intervals overlap -- for many regions at once.
-//
-// Mapping: one 128-thread block per (region, start) runs the whole EM of that start in fp64 -- for regions of many
-// samples (amplicon data: thousands of reads) a CLUSTER of 8 blocks whose partial sums meet through distributed shared
-// memory: every iteration is ONE pass over the region's bootstrapped sizes that computes the responsibilities (E step)
-// and accumulates the M step's three sums per component, followed by a fixed-order reduction (warps, block, cluster
-// ranks: results do not depend on scheduling).  The stopping rule,
-// the regularisation and the choice among the starts are scikit-learn's (BaseMixture.fit_predict); the random draws are
-// not: the reference uses unseeded generators (random.gauss, sklearn's k-means), this file a counter-based one
-// (splitmix64 of (seed, region, stream, index)) that the CPU checker shares -- a phased region is reproducible, and
-// independent of how regions are batched.  C ABI: nr_gmm_bootstrap, nr_gmm1d_fit, nr_phase_1d.
+// [isf(1 - o), isf(o)] intervals overlap -- for many regions at once, on the kernels of nr_launch_gmm.cu.  The stopping
+// rule, the regularisation and the choice among the starts are scikit-learn's (BaseMixture.fit_predict); the random
+// draws are not: the reference uses unseeded generators (random.gauss, sklearn's k-means), this library a counter-based
+// one that the CPU checker shares -- a phased region is reproducible, and independent of how regions are batched.
+// C ABI: nr_gmm_bootstrap, nr_gmm1d_fit, nr_phase_1d.
 #include "nr_internal.h"
+#include "nr_launch_gmm.h"
 
-#include <cooperative_groups.h>
 #include <algorithm>
 #include <cmath>
-#include <cstdio>
-#include <cstdlib>
 #include <vector>
 
-namespace cg = cooperative_groups;
+using namespace nrg;
 
 namespace {
-
-#define GTRY(expr)                                                                                       \
-    do {                                                                                                 \
-        cudaError_t e__ = (expr);                                                                        \
-        if (e__ != cudaSuccess) {                                                                        \
-            char b__[256];                                                                               \
-            snprintf(b__, sizeof b__, "%s failed: %s (%s:%d)", #expr, cudaGetErrorString(e__), __FILE__, __LINE__); \
-            return nri::fail_msg(NR_ERR_CUDA, b__);                                                      \
-        }                                                                                                \
-    } while (0)
-
-constexpr int kMaxC = NR_GMM_MAX_COMPONENTS;      // components per mixture
-constexpr int kThreads = 128;
-constexpr int kBootstrap = 100;                   // split_alleles.py:83
-constexpr int kLloyd = 10;
-constexpr int kBigCluster = 8;                    // thread blocks per fit for regions of many samples (portable cluster size)
-constexpr int kBigSamples = 16384;                // ... from this many bootstrapped samples on
-constexpr double kLog2Pi = 1.8378770664093453;    // log(2 pi)
-constexpr double kEps10 = 10 * 2.220446049250313e-16;
-
-struct Problem {          // one mixture fit: data[off .. off + count), n components
-    long long off;
-    long long region;     // stream id of the random draws
-    int count, n;
-};
-
-struct Fit {              // result of one (problem, start)
-    double lower;
-    int iters, converged;
-    double w[kMaxC], m[kMaxC], v[kMaxC];
-};
-
-__host__ __device__ inline unsigned long long mix64(unsigned long long x) {
-    x += 0x9E3779B97F4A7C15ull;
-    x = (x ^ (x >> 30)) * 0xBF58476D1CE4E5B9ull;
-    x = (x ^ (x >> 27)) * 0x94D049BB133111EBull;
-    return x ^ (x >> 31);
-}
-__host__ __device__ inline unsigned long long key(unsigned long long seed, long long region, unsigned long long stream, unsigned long long idx) {
-    return mix64(mix64(mix64(seed ^ (0xD1B54A32D192ED03ull * (unsigned long long)(region + 1))) + stream) + idx);
-}
-__device__ inline double uniform01(unsigned long long h) { return (double)((h >> 11) + 1) * (1.0 / 9007199254740992.0); }
-
-// sample rep * n + i of a region = x[i] + N(0, error_rate * (10 + x[i]))       (split_alleles.py:82-88)
-__global__ void bootstrap_kernel(const double* __restrict__ sizes, const long long* __restrict__ off, int n_regions, long long region_base,
-                                 double error_rate, unsigned long long seed, double* __restrict__ out) {
-    for (int g = blockIdx.x; g < n_regions; g += gridDim.x) {
-        const long long o = off[g], n = off[g + 1] - o;
-        for (long long t = threadIdx.x; t < n * kBootstrap; t += blockDim.x) {
-            const double x = sizes[o + t % n];
-            const double u1 = uniform01(key(seed, region_base + g, 1, (unsigned long long)t));
-            const double u2 = uniform01(key(seed, region_base + g, 2, (unsigned long long)t));
-            const double z = sqrt(-2.0 * log(u1)) * cos(2.0 * 3.14159265358979323846 * u2);
-            out[o * kBootstrap + t] = x + error_rate * (10.0 + x) * z;
-        }
-    }
-}
-
-constexpr int kVals = 3 * kMaxC + 2;
-
-// Sum of v[0..n) over every thread of the CLUSTER (the thread blocks that share one fit), in a fixed order: warps by
-// shuffle, the block's warps in shared memory, the cluster's blocks by rank through distributed shared memory.  Every
-// thread of every block may read tot[0..n) afterwards (all blocks hold the same totals, computed in the same order).
-__device__ inline void cluster_sum(cg::cluster_group& cluster, double* v, int n, double* red /* [4][kVals] */, double* tot /* [kVals] */) {
-    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-    for (int i = 0; i < n; ++i) {
-        double x = v[i];
-#pragma unroll
-        for (int o = 16; o > 0; o >>= 1) x += __shfl_xor_sync(0xffffffffu, x, o);
-        if (lane == 0) red[warp * kVals + i] = x;
-    }
-    __syncthreads();
-    if (threadIdx.x < n) {
-        double s = 0;
-        for (int w = 0; w < kThreads / 32; ++w) s += red[w * kVals + threadIdx.x];
-        red[threadIdx.x] = s;                       // (row 0 of warp 0 is overwritten by its own column's total)
-    }
-    const unsigned nb = cluster.num_blocks();
-    if (nb == 1) {
-        __syncthreads();
-        if (threadIdx.x < n) tot[threadIdx.x] = red[threadIdx.x];
-        __syncthreads();
-        return;
-    }
-    cluster.sync();                                 // every block's partial sums are in its red[0..n)
-    if (threadIdx.x < n) {
-        double s = 0;
-        for (unsigned r = 0; r < nb; ++r) s += cluster.map_shared_rank(red, r)[threadIdx.x];
-        tot[threadIdx.x] = s;
-    }
-    cluster.sync();                                 // nobody overwrites red while a neighbour still reads it
-}
-
-// One fit = one cluster of thread blocks (one block for small regions, kBigCluster for regions of many samples):
-// cluster `blockIdx.x / cluster size` is (problem, start).  Every block of the cluster walks its share of the samples,
-// the sums meet in cluster_sum, and every block then updates the same parameters redundantly (no broadcast).
-__global__ void __launch_bounds__(kThreads)
-fit_kernel(const Problem* __restrict__ problems, const double* __restrict__ data, int n_init, int max_iter, double tol, double reg_covar,
-           unsigned long long seed, Fit* __restrict__ fits) {
-    cg::cluster_group cluster = cg::this_cluster();
-    const int nb = (int)cluster.num_blocks(), rank = (int)cluster.block_rank();
-    const int fit = (int)(blockIdx.x / nb);
-    __shared__ double red[(kThreads / 32) * kVals];
-    __shared__ double tot[kVals];
-    __shared__ double sw[kMaxC], sm[kMaxC], sv[kMaxC], spc[kMaxC], sc0[kMaxC];
-    const Problem pb = problems[fit / n_init];
-    const int init = fit % n_init, n = pb.n, N = pb.count;
-    const double* x = data + pb.off;
-    const int first = rank * kThreads + (int)threadIdx.x, stride = nb * kThreads;      // this thread's samples
-    double acc[kVals];
-
-    // ---- start: means (init 0: evenly over [min, max]; else hashed sample positions), kLloyd rounds of 1-D k-means
-    if (init == 0) {
-        double lo = 1e300, hi = -1e300;
-        for (int i = first; i < N; i += stride) { lo = fmin(lo, x[i]); hi = fmax(hi, x[i]); }
-#pragma unroll
-        for (int o = 16; o > 0; o >>= 1) { lo = fmin(lo, __shfl_xor_sync(0xffffffffu, lo, o)); hi = fmax(hi, __shfl_xor_sync(0xffffffffu, hi, o)); }
-        if ((threadIdx.x & 31) == 0) { red[threadIdx.x >> 5] = lo; red[4 + (threadIdx.x >> 5)] = hi; }
-        __syncthreads();
-        if (threadIdx.x == 0) {
-            red[8] = fmin(fmin(red[0], red[1]), fmin(red[2], red[3]));
-            red[9] = fmax(fmax(red[4], red[5]), fmax(red[6], red[7]));
-        }
-        if (nb > 1) cluster.sync(); else __syncthreads();
-        lo = 1e300; hi = -1e300;
-        for (int r = 0; r < nb; ++r) {
-            const double* rr = nb > 1 ? cluster.map_shared_rank(red, r) : red;
-            lo = fmin(lo, rr[8]); hi = fmax(hi, rr[9]);
-        }
-        if (nb > 1) cluster.sync(); else __syncthreads();
-        if (threadIdx.x < n) sm[threadIdx.x] = lo + (threadIdx.x + 0.5) / n * (hi - lo);
-    } else if (threadIdx.x < n) {
-        sm[threadIdx.x] = x[key(seed, pb.region, 1000 + 32 * n + init, threadIdx.x) % (unsigned long long)N];
-    }
-    __syncthreads();
-    for (int round = 0; round <= kLloyd; ++round) {
-        // labels by the nearest mean (lowest index on ties); the last round turns them into the first M step
-        for (int j = 0; j < 3 * n; ++j) acc[j] = 0;
-        for (int i = first; i < N; i += stride) {
-            const double xi = x[i];
-            int lab = 0;
-            double bd = fabs(xi - sm[0]);
-            for (int j = 1; j < n; ++j) { const double d = fabs(xi - sm[j]); if (d < bd) { bd = d; lab = j; } }
-            acc[lab] += 1.0; acc[n + lab] += xi; acc[2 * n + lab] += xi * xi;
-        }
-        cluster_sum(cluster, acc, 3 * n, red, tot);
-        if (threadIdx.x < n) {
-            const int j = threadIdx.x;
-            if (round < kLloyd) {
-                if (tot[j] > 0) sm[j] = tot[n + j] / tot[j];
-            } else {          // sklearn _estimate_gaussian_parameters on one-hot responsibilities
-                const double nk = tot[j] + kEps10;
-                const double mean = tot[n + j] / nk;
-                sw[j] = nk / N; sm[j] = mean; sv[j] = tot[2 * n + j] / nk - mean * mean + reg_covar;
-            }
-        }
-        __syncthreads();
-    }
-
-    // ---- EM (BaseMixture.fit_predict: E step, M step, |change of the mean log-likelihood| < tol)
-    double lower = -INFINITY;
-    int iters = 0, converged = 0;
-    for (int it = 1; it <= max_iter; ++it) {
-        if (threadIdx.x < n) {
-            const int j = threadIdx.x;
-            const double pc = 1.0 / sqrt(sv[j]);
-            spc[j] = pc;
-            sc0[j] = log(pc) + log(sw[j]) - 0.5 * kLog2Pi;
-        }
-        __syncthreads();
-        for (int j = 0; j < 3 * n + 1; ++j) acc[j] = 0;
-        for (int i = first; i < N; i += stride) {
-            const double xi = x[i];
-            double lp[kMaxC];
-            double top = -INFINITY;
-            for (int j = 0; j < n; ++j) {
-                const double d = (xi - sm[j]) * spc[j];
-                lp[j] = sc0[j] - 0.5 * d * d;
-                top = fmax(top, lp[j]);
-            }
-            double s = 0;
-            for (int j = 0; j < n; ++j) s += exp(lp[j] - top);
-            const double norm = top + log(s);
-            for (int j = 0; j < n; ++j) {
-                const double r = exp(lp[j] - norm);
-                acc[j] += r; acc[n + j] += r * xi; acc[2 * n + j] += r * xi * xi;
-            }
-            acc[3 * n] += norm;
-        }
-        cluster_sum(cluster, acc, 3 * n + 1, red, tot);
-        const double prev = lower;
-        lower = tot[3 * n] / N;
-        __syncthreads();
-        if (threadIdx.x < n) {
-            const int j = threadIdx.x;
-            const double nk = tot[j] + kEps10;
-            const double mean = tot[n + j] / nk;
-            sw[j] = nk / N; sm[j] = mean; sv[j] = tot[2 * n + j] / nk - mean * mean + reg_covar;
-        }
-        __syncthreads();
-        iters = it;
-        if (fabs(lower - prev) < tol) { converged = 1; break; }        // (the same number in every block: all leave together)
-    }
-    if (rank == 0) {
-        Fit& f = fits[fit];
-        if (threadIdx.x == 0) { f.lower = lower; f.iters = iters; f.converged = converged; }
-        if (threadIdx.x < n) { f.w[threadIdx.x] = sw[threadIdx.x]; f.m[threadIdx.x] = sm[threadIdx.x]; f.v[threadIdx.x] = sv[threadIdx.x]; }
-    }
-}
-
-struct Bufs {
-    struct One { void* p; size_t bytes; bool pinned; };
-    std::vector<One> all;
-    int get(void** p, size_t bytes, bool pinned) {
-        *p = nullptr;
-        const int rc = nri::alloc(p, std::max<size_t>(bytes, 16), pinned);
-        if (rc == NR_OK) all.push_back({*p, std::max<size_t>(bytes, 16), pinned});
-        return rc;
-    }
-    ~Bufs() { for (const One& b : all) nri::release(b.p, b.bytes, b.pinned); }
-};
 
 int check_params(const nr_gmm_params_t* p) {
     if (!p || p->max_components < 1 || p->max_components > kMaxC || p->n_init < 1 || p->n_init > 64 || p->max_iter < 1 ||
         !(p->tol > 0) || !(p->reg_covar >= 0) || !(p->error_rate >= 0) || !(p->max_mutual_overlap > 0 && p->max_mutual_overlap < 1))
-        return nri::fail_msg(NR_ERR_ARG, "nr_gmm: bad parameters (1 <= max_components <= NR_GMM_MAX_COMPONENTS, 1 <= n_init <= 64, 0 < overlap < 1)");
+        return nri::fail(NR_ERR_ARG, "nr_gmm: bad parameters (1 <= max_components <= NR_GMM_MAX_COMPONENTS, 1 <= n_init <= 64, 0 < overlap < 1)");
     return NR_OK;
 }
 
@@ -277,7 +48,7 @@ int run_fits(const nr_gmm_params_t* p, const std::vector<Problem>& problems, con
     best.resize(np);
     if (np == 0) return NR_OK;
     const size_t n_fits = (size_t)np * p->n_init;
-    Bufs bufs;
+    nri::Bufs bufs;
     void *d_prob = nullptr, *d_fits = nullptr, *h_fits = nullptr;
     int rc;
     if ((rc = bufs.get(&d_prob, sizeof(Problem) * np, false)) || (rc = bufs.get(&d_fits, sizeof(Fit) * n_fits, false)) ||
@@ -292,27 +63,12 @@ int run_fits(const nr_gmm_params_t* p, const std::vector<Problem>& problems, con
     while (n_small < np && problems[perm[n_small]].count < kBigSamples) ++n_small;
     std::vector<Problem> sorted(np);
     for (int i = 0; i < np; ++i) sorted[i] = problems[perm[i]];
-    GTRY(cudaMemcpyAsync(d_prob, sorted.data(), sizeof(Problem) * np, cudaMemcpyHostToDevice, st));
-    auto launch = [&](int first, int count, int cluster) -> cudaError_t {
-        if (count == 0) return cudaSuccess;
-        cudaLaunchConfig_t cfg = {};
-        cfg.gridDim = dim3((unsigned)((size_t)count * p->n_init * cluster));
-        cfg.blockDim = dim3(kThreads);
-        cfg.dynamicSmemBytes = 0;
-        cfg.stream = st;
-        cudaLaunchAttribute attr[1];
-        attr[0].id = cudaLaunchAttributeClusterDimension;
-        attr[0].val.clusterDim.x = (unsigned)cluster; attr[0].val.clusterDim.y = 1; attr[0].val.clusterDim.z = 1;
-        cfg.attrs = attr;
-        cfg.numAttrs = 1;
-        return cudaLaunchKernelEx(&cfg, fit_kernel, static_cast<const Problem*>(d_prob) + first, d_data, (int)p->n_init, (int)p->max_iter,
-                                  (double)p->tol, (double)p->reg_covar, (unsigned long long)p->seed,
-                                  static_cast<Fit*>(d_fits) + (size_t)first * p->n_init);
-    };
-    GTRY(launch(0, n_small, 1));
-    GTRY(launch(n_small, np - n_small, kBigCluster));
-    GTRY(cudaMemcpyAsync(h_fits, d_fits, sizeof(Fit) * n_fits, cudaMemcpyDeviceToHost, st));
-    GTRY(cudaStreamSynchronize(st));
+    CUDA_TRY(cudaMemcpyAsync(d_prob, sorted.data(), sizeof(Problem) * np, cudaMemcpyHostToDevice, st));
+    CUDA_TRY(nrl::launch_gmm_fits(*p, n_small, 1, st, static_cast<const Problem*>(d_prob), d_data, static_cast<Fit*>(d_fits)));
+    CUDA_TRY(nrl::launch_gmm_fits(*p, np - n_small, kBigCluster, st, static_cast<const Problem*>(d_prob) + n_small, d_data,
+                                  static_cast<Fit*>(d_fits) + (size_t)n_small * p->n_init));
+    CUDA_TRY(cudaMemcpyAsync(h_fits, d_fits, sizeof(Fit) * n_fits, cudaMemcpyDeviceToHost, st));
+    CUDA_TRY(cudaStreamSynchronize(st));
     const Fit* f = static_cast<const Fit*>(h_fits);
     for (int s = 0; s < np; ++s) {
         const int i = perm[s];
@@ -332,7 +88,7 @@ int run_fits(const nr_gmm_params_t* p, const std::vector<Problem>& problems, con
 }
 
 int upload_and_bootstrap(const nr_gmm_params_t* p, int n_regions, const std::vector<long long>& off, const double* sizes, long long region_base,
-                         Bufs& bufs, double** d_sim) {
+                         nri::Bufs& bufs, double** d_sim) {
     const long long total = off[n_regions];
     void *d_sizes = nullptr, *d_off = nullptr, *sim = nullptr;
     int rc;
@@ -340,12 +96,11 @@ int upload_and_bootstrap(const nr_gmm_params_t* p, int n_regions, const std::vec
         (rc = bufs.get(&sim, sizeof(double) * total * kBootstrap, false)))
         return rc;
     cudaStream_t st = nri::stream();
-    GTRY(cudaMemcpyAsync(d_sizes, sizes, sizeof(double) * total, cudaMemcpyHostToDevice, st));
-    GTRY(cudaMemcpyAsync(d_off, off.data(), sizeof(long long) * (n_regions + 1), cudaMemcpyHostToDevice, st));
+    CUDA_TRY(cudaMemcpyAsync(d_sizes, sizes, sizeof(double) * total, cudaMemcpyHostToDevice, st));
+    CUDA_TRY(cudaMemcpyAsync(d_off, off.data(), sizeof(long long) * (n_regions + 1), cudaMemcpyHostToDevice, st));
     const int blocks = std::max(1, std::min(n_regions, 8 * nri::sm_count()));
-    bootstrap_kernel<<<blocks, 256, 0, st>>>(static_cast<const double*>(d_sizes), static_cast<const long long*>(d_off), n_regions, region_base,
-                                            p->error_rate, p->seed, static_cast<double*>(sim));
-    GTRY(cudaGetLastError());
+    CUDA_TRY(nrl::launch_gmm_bootstrap(*p, blocks, st, static_cast<const double*>(d_sizes), static_cast<const long long*>(d_off), n_regions,
+                                       region_base, static_cast<double*>(sim)));
     *d_sim = static_cast<double*>(sim);
     return NR_OK;
 }
@@ -355,18 +110,18 @@ int upload_and_bootstrap(const nr_gmm_params_t* p, int n_regions, const std::vec
 extern "C" int nr_gmm_bootstrap(const nr_gmm_params_t* p, int32_t n_regions, const int64_t* offsets, const double* sizes,
                                 int64_t region_id_base, double* out) {
     if (check_params(p)) return nri::last_code();
-    if (n_regions < 0 || (n_regions > 0 && (!offsets || !sizes || !out))) return nri::fail_msg(NR_ERR_ARG, "nr_gmm_bootstrap: bad arguments");
+    if (n_regions < 0 || (n_regions > 0 && (!offsets || !sizes || !out))) return nri::fail(NR_ERR_ARG, "nr_gmm_bootstrap: bad arguments");
     int rc = nri::ensure_init();
     if (rc || n_regions == 0) return rc;
     std::vector<long long> off(offsets, offsets + n_regions + 1);
     for (int g = 0; g < n_regions; ++g)
-        if (off[g + 1] < off[g] || off[0] != 0) return nri::fail_msg(NR_ERR_ARG, "nr_gmm_bootstrap: offsets must start at 0 and not decrease");
+        if (off[g + 1] < off[g] || off[0] != 0) return nri::fail(NR_ERR_ARG, "nr_gmm_bootstrap: offsets must start at 0 and not decrease");
     if (off[n_regions] == 0) return NR_OK;
-    Bufs bufs;
+    nri::Bufs bufs;
     double* d_sim = nullptr;
     if ((rc = upload_and_bootstrap(p, n_regions, off, sizes, region_id_base, bufs, &d_sim))) return rc;
-    GTRY(cudaMemcpyAsync(out, d_sim, sizeof(double) * off[n_regions] * kBootstrap, cudaMemcpyDeviceToHost, nri::stream()));
-    GTRY(cudaStreamSynchronize(nri::stream()));
+    CUDA_TRY(cudaMemcpyAsync(out, d_sim, sizeof(double) * off[n_regions] * kBootstrap, cudaMemcpyDeviceToHost, nri::stream()));
+    CUDA_TRY(cudaStreamSynchronize(nri::stream()));
     return NR_OK;
 }
 
@@ -375,20 +130,20 @@ extern "C" int nr_gmm1d_fit(const nr_gmm_params_t* p, int32_t n_problems, const 
                             double* weights, double* means, double* variances) {
     if (check_params(p)) return nri::last_code();
     if (n_problems < 0 || (n_problems > 0 && (!offsets || !data || !n_components || !weights || !means || !variances)))
-        return nri::fail_msg(NR_ERR_ARG, "nr_gmm1d_fit: bad arguments");
+        return nri::fail(NR_ERR_ARG, "nr_gmm1d_fit: bad arguments");
     int rc = nri::ensure_init();
     if (rc || n_problems == 0) return rc;
     std::vector<Problem> problems(n_problems);
     for (int i = 0; i < n_problems; ++i) {
         const long long cnt = offsets[i + 1] - offsets[i];
         if (offsets[0] != 0 || cnt < 1 || cnt > 0x7fffffff || n_components[i] < 1 || n_components[i] > p->max_components)
-            return nri::fail_msg(NR_ERR_ARG, "nr_gmm1d_fit: every problem needs >= 1 sample and 1 <= n_components <= max_components");
+            return nri::fail(NR_ERR_ARG, "nr_gmm1d_fit: every problem needs >= 1 sample and 1 <= n_components <= max_components");
         problems[i] = {offsets[i], region_id ? region_id[i] : i, (int)cnt, n_components[i]};
     }
-    Bufs bufs;
+    nri::Bufs bufs;
     void* d_data = nullptr;
     if ((rc = bufs.get(&d_data, sizeof(double) * offsets[n_problems], false))) return rc;
-    GTRY(cudaMemcpyAsync(d_data, data, sizeof(double) * offsets[n_problems], cudaMemcpyHostToDevice, nri::stream()));
+    CUDA_TRY(cudaMemcpyAsync(d_data, data, sizeof(double) * offsets[n_problems], cudaMemcpyHostToDevice, nri::stream()));
     std::vector<Fit> best;
     if ((rc = run_fits(p, problems, static_cast<const double*>(d_data), best))) return rc;
     for (int i = 0; i < n_problems; ++i) {
@@ -409,12 +164,12 @@ extern "C" int nr_phase_1d(const nr_gmm_params_t* p, int32_t n_regions, const in
                            int32_t* label, double* proba) {
     if (check_params(p)) return nri::last_code();
     if (n_regions < 0 || (n_regions > 0 && (!offsets || !n_components || !weights || !means || !variances)))
-        return nri::fail_msg(NR_ERR_ARG, "nr_phase_1d: bad arguments");
+        return nri::fail(NR_ERR_ARG, "nr_phase_1d: bad arguments");
     int rc = nri::ensure_init();
     if (rc || n_regions == 0) return rc;
-    if (offsets[0] != 0) return nri::fail_msg(NR_ERR_ARG, "nr_phase_1d: offsets must start at 0");
+    if (offsets[0] != 0) return nri::fail(NR_ERR_ARG, "nr_phase_1d: offsets must start at 0");
     const long long total = offsets[n_regions];
-    if (total > 0 && (!sizes || !label || !proba)) return nri::fail_msg(NR_ERR_ARG, "nr_phase_1d: bad arguments");
+    if (total > 0 && (!sizes || !label || !proba)) return nri::fail(NR_ERR_ARG, "nr_phase_1d: bad arguments");
     const int C = p->max_components;
     for (long long i = 0; i < total; ++i) { label[i] = -1; proba[i] = 0.0; }
     for (size_t i = 0; i < (size_t)n_regions * C; ++i) weights[i] = means[i] = variances[i] = 0.0;
@@ -428,10 +183,10 @@ extern "C" int nr_phase_1d(const nr_gmm_params_t* p, int32_t n_regions, const in
     kept_src.reserve((size_t)total);
     for (int g = 0; g < n_regions; ++g) {
         const long long a = offsets[g], b = offsets[g + 1];
-        if (b < a) return nri::fail_msg(NR_ERR_ARG, "nr_phase_1d: offsets must not decrease");
+        if (b < a) return nri::fail(NR_ERR_ARG, "nr_phase_1d: offsets must not decrease");
         n_components[g] = 0;
         if (b - a >= 2) {
-            if ((b - a) * (long long)kBootstrap > 0x7fffffff) return nri::fail_msg(NR_ERR_TOO_LARGE, "nr_phase_1d: more than 21 million sizes in one region");
+            if ((b - a) * (long long)kBootstrap > 0x7fffffff) return nri::fail(NR_ERR_TOO_LARGE, "nr_phase_1d: more than 21 million sizes in one region");
             double s = 0;
             for (long long i = a; i < b; ++i) s += sizes[i];
             const double mean = s / (double)(b - a);
@@ -446,7 +201,7 @@ extern "C" int nr_phase_1d(const nr_gmm_params_t* p, int32_t n_regions, const in
     }
     if (kept.empty()) return NR_OK;
 
-    Bufs bufs;
+    nri::Bufs bufs;
     double* d_sim = nullptr;
     if ((rc = upload_and_bootstrap(p, n_regions, toff, kept.data(), region_id_base, bufs, &d_sim))) return rc;
 

@@ -97,7 +97,7 @@ struct Planner {
                 continue;
             }
             long long m = (long long)b->sc.match * std::min(q_len, t_len);
-            if (m > kMaxScore || t_len > kMaxTlen) {        // (its cells stay in the count of what was asked for)
+            if (m > nri::kMaxScore || t_len > kMaxTlen) {   // (its cells stay in the count of what was asked for)
                 paired[i] = 2;
                 ++b->n_skipped;
                 continue;
@@ -201,7 +201,7 @@ struct Planner {
             });
             i0 = i1;
         }
-        if (rung_off > 0x7fffffffLL) return fail(NR_ERR_TOO_LARGE, "more than 2^31 rungs in one batch");
+        if (rung_off > 0x7fffffffLL) return nri::fail(NR_ERR_TOO_LARGE, "more than 2^31 rungs in one batch");
         L.redo_R = L.pair_R;
         return NR_OK;
     }
@@ -307,7 +307,7 @@ struct Planner {
                 if (stripes(q_len(i), R) > nr::kCodeFwd - 2)        // too long for that many stripes: its own, taller ones
                     R = nr::coop_height_at_least(nr::coop_rows(q_len(i), nr::kCodeFwd - 2));
                 if (R > max_r)
-                    return fail(NR_ERR_TOO_LARGE, "task %d: a query of %d bases needs more than %d stripes", i, q_len(i), nr::kCodeFwd - 2);
+                    return nri::fail(NR_ERR_TOO_LARGE, "task %d: a query of %d bases needs more than %d stripes", i, q_len(i), nr::kCodeFwd - 2);
                 restripe(i, R);
             }
         }
@@ -344,7 +344,7 @@ struct Planner {
         ci.flag_off = (int)flag_off;
         data_off += words;
         flag_off += nr::kCoopFlagInts(ci.n_stripes);
-        if (flag_off > 0x7fffffffLL) return fail(NR_ERR_TOO_LARGE, "too many long tasks in one batch");
+        if (flag_off > 0x7fffffffLL) return nri::fail(NR_ERR_TOO_LARGE, "too many long tasks in one batch");
         b->coop.push_back(ci);
         return NR_OK;
     }
@@ -410,12 +410,12 @@ struct Planner {
         auto by_cost = [&](int x, int y) { return cost[x] != cost[y] ? cost[x] > cost[y] : x < y; };
         std::sort(singles.begin(), singles.end(), by_cost);
         std::sort(multis.begin(), multis.end(), by_cost);
-        if (n > (1 << (31 - nr::kCodeBits))) return fail(NR_ERR_TOO_LARGE, "more than 2^24 tasks in one batch");
+        if (n > (1 << (31 - nr::kCodeBits))) return nri::fail(NR_ERR_TOO_LARGE, "more than 2^24 tasks in one batch");
         b->order.clear();
         b->coop.clear();
         int rc;
         if ((rc = coop_layout())) return rc;
-        if (rung_off > 0x7fffffffLL) return fail(NR_ERR_TOO_LARGE, "more than 2^31 rungs in one batch");
+        if (rung_off > 0x7fffffffLL) return nri::fail(NR_ERR_TOO_LARGE, "more than 2^31 rungs in one batch");
         if (!b->pairs3.empty()) b->prung_bytes = sizeof(uint2) * (size_t)std::max<long long>(rung_off, 1);
         // Stripe-major: stripe 0 of every long task, then stripe 1 of every long task, ...  A stripe waits for the one
         // above it; listed task by task, all stripes of a task would be picked up at the same moment and stripe s would
@@ -482,7 +482,7 @@ struct Planner {
 // launches and the buffers.
 int plan_batch(nr_batch* b, int sm_count) {
     Planner p{b, sm_count};
-    PhaseTrace trace;
+    nri::PhaseTrace trace;
     int rc;
     p.task_shapes();
     trace.mark("task shapes");

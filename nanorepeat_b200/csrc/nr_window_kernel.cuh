@@ -27,32 +27,13 @@
 // scratch row in global memory (L2), read back 32 columns at a time.  The wavefront is skewed (lane l works on column
 // step - l) and the bottom row moves down the lanes by shuffle, as in nr_kernels.cuh.
 #pragma once
-#include <cuda_runtime.h>
-#include <stdint.h>
+#include "nr_launch_window.h"
 #include <type_traits>
 
 namespace nrw {
 
-struct WinTask {           // 32 bytes
-    uint32_t q_word;       // 2-bit packed read (same pool layout as nr_kernels.cuh, ambiguity plane included)
-    int32_t  q_len;
-    uint32_t t_word;       // 2-bit packed template
-    int32_t  t_len;
-    int32_t  win_a, win_b; // window [a, b) in template coordinates
-    int32_t  reverse;      // 1: align the reverse complement of the read
-    int32_t  pad;
-};
-
-constexpr int kR = 8;                  // rows per lane
-constexpr int kRows = 32 * kR;         // rows per stripe
-constexpr int kWarps = 8;              // warps per block
 constexpr unsigned kFull = 0xffffffffu;
 constexpr int kPad = -(16384 << 16);
-
-struct WinScore {          // scoring as word increments (upper half: alignment score)
-    int match, mismatch, ambiguous;          // a << 16, -(b << 16), -(sc_ambi << 16)
-    int open1, ext1, open2, ext2;            // -((q + e) << 16), -(e << 16), ...
-};
 
 __device__ __forceinline__ bool amb_base(const uint32_t* __restrict__ q, uint32_t plane, int i) {
     return plane && ((q[plane + (i >> 5)] >> (i & 31)) & 1u);

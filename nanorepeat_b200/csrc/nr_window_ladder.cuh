@@ -37,40 +37,6 @@
 
 namespace nrw {
 
-struct LadBwdTask {        // one per (read, strand)
-    uint32_t q_word; int32_t q_len;
-    uint32_t rev_word; int32_t n_right;    // reverse(right)
-    int32_t reverse;                       // strand
-    int32_t pad;
-    // First word of this task's junction vectors (3 planes of q_len words).  64-bit: a call spends 6 words per read base
-    // on the shared path, past 2^31 after ~358 M bases.  Kept as two 32-bit halves: a long long member makes the struct
-    // 8-byte aligned, and ptxas then gives both ladder kernels 128 registers (64 / 80 with the halves) and a spill.
-    uint32_t bvec_lo, bvec_hi;
-    __host__ __device__ long long bvec_off() const { return (long long)(((unsigned long long)bvec_hi << 32) | bvec_lo); }
-    void set_bvec_off(long long w) { bvec_lo = (uint32_t)w; bvec_hi = (uint32_t)((unsigned long long)w >> 32); }
-};
-static_assert(sizeof(LadBwdTask) == 32, "LadBwdTask is 32 bytes");
-
-struct LadFwdTask {        // one per (read, strand, k1)
-    uint32_t q_word; int32_t q_len;
-    uint32_t t_word;                       // left + motif1*k1 + mid + motif2*k2max(of the locus)
-    int32_t n_pre;                         // |left| + m1*k1 + |mid|: columns before the second repeat
-    int32_t m2, k2_first, k2_step, k2_count;
-    int32_t win_a;                         // |left| - 10 (>= 0)
-    int32_t reverse;
-    int32_t bwd;                           // index of the (read, strand)'s LadBwdTask
-    int32_t out_off;                       // first record of this task in out[]: k2_count records (prefix: in pbest1[])
-    int32_t mode;                          // kWhole / kPrefix / kCont
-    int32_t pbest1;                        // kCont: index into pbest1[] of this k1's entry
-    long long cstate;                      // kPrefix: first word of its saved columns [k][3][q_len]; kCont: of its own column
-};
-// kWhole: the whole forward template from the empty column.  kPrefix: the fields n_pre / m2 / k2_* describe the k1
-// junctions (n_pre = |left|, m2 = m1, ...); nothing is joined, states are saved.  kCont: t_word = mid + motif2*k2max,
-// n_pre = |mid|, every column inside the window.
-constexpr int kWhole = 0, kPrefix = 1, kCont = 2;
-
-constexpr int kMaxK2 = 64;                 // grid points per forward task (shared-memory tables)
-
 // Substitution words of one stripe for the oriented read (strand: reverse complement), optionally walked backwards
 // (backward sweep).  prof[(win * 4 + c) * kRows + lane * kR + r].
 __device__ __forceinline__ void build_profile2(int* prof, const uint32_t* __restrict__ q, int q_len, bool strand, bool backwards,
