@@ -372,6 +372,35 @@ int nr_gmm1d_fit(const nr_gmm_params_t* p, int32_t n_problems, const int64_t* of
                  const int32_t* n_components, const int64_t* region_id, double* lower, int32_t* iters,
                  double* weights, double* means, double* variances);
 
+/* ---- Mixture fits of one or two features per sample ---------------------------------------------------------------
+ * What scikit-learn's GaussianMixture(n_components, covariance_type='diag', tol, reg_covar, max_iter, n_init).fit does,
+ * for many problems in one call: problem i is samples data[offsets[i] .. offsets[i + 1]), sample-major with n_features
+ * (1 or 2) values each, fitted with n_components[i] components.  fp64 EM with scikit-learn's E / M steps, regularisation,
+ * stopping rule (|change of the mean log-likelihood| < tol, max_iter at most) and choice among the starts (the first of
+ * the highest lower bounds); weights come back as nk / n_samples (scikit-learn divides by the sum of nk, which differs by
+ * n_components * 10 eps / n_samples relative).  p->max_components is the output stride; p->error_rate and
+ * p->max_mutual_overlap are not used.
+ *   Starts.  weights_init [i * max_components + j], means_init and precisions_init [(i * max_components + j) * n_features
+ * + d] given (all three, or none): one start per problem from these parameters (scikit-learn's n_init starts would all be
+ * the same).  None given: p->n_init starts per problem from the library's k-means stand-in, keyed by (p->seed,
+ * region_id[i] or i): start 0 puts the means evenly along the samples' bounding box, lo_d + (j + 1/2) / n (hi_d - lo_d);
+ * start s > 0 takes the sample rows key(seed, region, 1000 + 32 n + s, j) mod count; then 10 Lloyd rounds on the squared
+ * Euclidean distance (first index on a tie) and the M step of the one-hot labels.  At n_features = 1 this is
+ * nr_gmm1d_fit's start, and a problem's result does not depend on the other problems of the call.
+ *   Output.  lower[i], iters[i], converged[i] (each nullable) and weights / means / variances in the layout of the
+ * starts, zero beyond n_components[i].  Components come in the fit's order, NOT sorted (scikit-learn does not sort them,
+ * and explicit starts keep theirs).
+ *   Pinned.  From explicit starts the fit equals scikit-learn to rounding (the CPU checker oracle/gmm_nd.py to 1e-9
+ * against scikit-learn, the device to 1e-7 against the checker).  From the k-means stand-in the device equals the checker,
+ * which shares its random draws; against scikit-learn's own k-means starts agreement is statistical.
+ *   NR_ERR_ARG: n_features not 1 or 2, n_components[i] not in [1, max_components] (at most NR_GMM_MAX_COMPONENTS), a
+ * problem with fewer samples than components, a sample that is not finite, or only some of the three starts given.
+ * nr_last_stats: n_tasks = problems x starts, kernel_launches. */
+int nr_gmm_fit(const nr_gmm_params_t* p, int32_t n_features, int32_t n_problems, const int64_t* offsets, const double* data,
+               const int32_t* n_components, const int64_t* region_id, const double* weights_init, const double* means_init,
+               const double* precisions_init, double* lower, int32_t* iters, uint8_t* converged, double* weights, double* means,
+               double* variances);
+
 /* Counters of the last nr_score_tasks / nr_round2_region / nr_round3_region / nr_window_tasks / nr_joint_grid call on
  * this thread. */
 int nr_last_stats(nr_stats_t* out);

@@ -137,6 +137,8 @@ SYMBOLS = {
     "nr_phase_1d": (ctypes.c_int, [_gmp, ctypes.c_int32, _i64p, _f64p, ctypes.c_int64, _i32p, _f64p, _f64p, _f64p, _i32p, _f64p]),
     "nr_gmm_bootstrap": (ctypes.c_int, [_gmp, ctypes.c_int32, _i64p, _f64p, ctypes.c_int64, _f64p]),
     "nr_gmm1d_fit": (ctypes.c_int, [_gmp, ctypes.c_int32, _i64p, _f64p, _i32p, _i64p, _f64p, _i32p, _f64p, _f64p, _f64p]),
+    "nr_gmm_fit": (ctypes.c_int, [_gmp, ctypes.c_int32, ctypes.c_int32, _i64p, _f64p, _i32p, _i64p, _f64p, _f64p, _f64p, _f64p,
+                                  _i32p, ctypes.c_void_p, _f64p, _f64p, _f64p]),
     "nr_estimate_regions": (ctypes.c_int, [_scp, ctypes.c_int32, ctypes.c_int32, ctypes.POINTER(RegionIn),
                                            ctypes.POINTER(ctypes.c_double), ctypes.POINTER(ctypes.c_double), ctypes.c_void_p,
                                            ctypes.POINTER(ctypes.c_double), ctypes.c_void_p, _i32p, ctypes.POINTER(Stats)]),
@@ -665,6 +667,44 @@ def gmm1d_fit(params, data_lists, n_components, region_ids=None):
                               iters.ctypes.data_as(_i32p), w.ctypes.data_as(_f64p), m.ctypes.data_as(_f64p), v.ctypes.data_as(_f64p)))
     return dict(lower=lower, iters=iters, weights=[w[i, :nc[i]] for i in range(n)], means=[m[i, :nc[i]] for i in range(n)],
                 variances=[v[i, :nc[i]] for i in range(n)])
+
+
+def gmm_fit(params, data_lists, n_components, n_features, region_ids=None, init=None):
+    """nr_gmm_fit: a diagonal-covariance mixture of n_components[i] components fitted to every problem's samples
+    (data_lists[i]: shape (N_i, n_features), or (N_i,) at one feature).  init: None (best of params.n_init starts of the
+    k-means stand-in) or (weights, means, precisions), one entry per problem of shapes (n,), (n, D), (n, D) (one start).
+    -> dict(lower, iters, converged, weights, means, variances), the last three as lists of arrays of shapes (n,), (n, D),
+    (n, D); components in the fit's order."""
+    D = int(n_features)
+    n = len(data_lists)
+    rows = [np.asarray(x, dtype=np.float64).reshape(-1, D) if D in (1, 2) else np.asarray(x, dtype=np.float64) for x in data_lists]
+    off = np.zeros(n + 1, dtype=np.int64)
+    if n:
+        np.cumsum([len(x) for x in rows], out=off[1:])
+    flat = np.ascontiguousarray(np.concatenate(rows).reshape(-1) if off[-1] else np.zeros(0))
+    nc = np.ascontiguousarray(n_components, dtype=np.int32)
+    if len(nc) != n:
+        raise ValueError("one n_components entry per problem")
+    rid = None if region_ids is None else np.ascontiguousarray(region_ids, dtype=np.int64)
+    C = params.max_components
+    starts = [None, None, None]
+    if init is not None:
+        wi, mi, pi = init
+        starts = [np.zeros((n, C)), np.zeros((n, C, max(D, 1))), np.ones((n, C, max(D, 1)))]
+        for i in range(n):
+            k = int(nc[i])
+            starts[0][i, :k] = np.asarray(wi[i], dtype=np.float64).reshape(k)
+            starts[1][i, :k] = np.asarray(mi[i], dtype=np.float64).reshape(k, D)
+            starts[2][i, :k] = np.asarray(pi[i], dtype=np.float64).reshape(k, D)
+    lower, iters, conv = np.zeros(n), np.zeros(n, dtype=np.int32), np.zeros(n, dtype=np.uint8)
+    w, m, v = np.zeros((n, C)), np.zeros((n, C, max(D, 1))), np.zeros((n, C, max(D, 1)))
+    _check(lib().nr_gmm_fit(ctypes.byref(params), D, n, off.ctypes.data_as(_i64p), flat.ctypes.data_as(_f64p), nc.ctypes.data_as(_i32p),
+                            None if rid is None else rid.ctypes.data_as(_i64p),
+                            *[None if a is None else a.ctypes.data_as(_f64p) for a in starts],
+                            lower.ctypes.data_as(_f64p), iters.ctypes.data_as(_i32p), conv.ctypes.data, w.ctypes.data_as(_f64p),
+                            m.ctypes.data_as(_f64p), v.ctypes.data_as(_f64p)))
+    return dict(lower=lower, iters=iters, converged=conv.astype(bool), weights=[w[i, :nc[i]] for i in range(n)],
+                means=[m[i, :nc[i]] for i in range(n)], variances=[v[i, :nc[i]] for i in range(n)])
 
 
 def phase_1d(params, size_lists, region_id_base=0):
